@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- dyad-timesteps/s of the Temporal-AME structured mean-field VI fit loop on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 4|3|n,T,r]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 4|3|n,T,r] [--dump-outputs DIR]
 
 One "step" = one iteration of fit(): a full Gauss-Seidel sweep + ELBO + reconstruction MSE ("good" SMF, FP64),
 i.e. n^2 * T dyad-timesteps.  At N GPUs the SAME problem is node-sharded (strong scaling).  Workload: BASELINE
@@ -14,6 +14,9 @@ is the oracle port timed on the host cores on a FIXED sample (CPU_SAMPLE_NODES n
 sample `--impl reference` times, so the two arms describe one configuration.  `extra` carries BASELINE configs 3
 (200 sweeps, three reciprocity values) and 5 (512 batched fits).  --impl reference also times the unmodified
 reference (copied to oracle/_ref at build time, when present) on BASELINE config 1.
+
+--dump-outputs DIR writes what the last timed step handed back (ELBO, its parts, MSE, the variational state) as
+float64 .npy files; the inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import ctypes as C
@@ -39,6 +42,7 @@ METRIC = "SMF-VI dyad-timesteps/sec (N^2*T per sweep; sweep + ELBO + MSE per ste
 UNIT = "dyad-timesteps/s"
 PANEL = int(os.environ.get("TAME_PANEL", "64"))    # nodes per ownership panel of the multi-GPU fit (multiple of 64)
 CPU_SAMPLE_NODES = 384      # fixed node subsample of the workload timed on the host (cpu_baseline and --impl reference)
+DUMP_STATE_BYTES = 60 << 20     # --dump-outputs: state rows kept so that all files together stay under 64 MB
 
 
 def parse_shape(s):
@@ -317,6 +321,23 @@ def init_state(n, T, d, dev, seed=42):
     return Xm, Xc
 
 
+def dump_outputs(path, Xm, Xc, out6):
+    """What one fit iteration returns to its caller: the ELBO, its four parts (expected log-likelihood, initial prior,
+    transition prior, entropy), the reconstruction MSE and the variational state, as float64 .npy files.  X_mean and
+    X_cov hold all nodes when they fit DUMP_STATE_BYTES, else a fixed, seeded sample of nodes (every time step of each);
+    node_index.npy lists which."""
+    import torch
+    n, T, d = Xm.shape
+    k = min(n, DUMP_STATE_BYTES // (T * d * (d + 1) * 8))
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    sel = torch.from_numpy(idx).to(Xm.device)
+    arrays = {"elbo": out6[0], "elbo_parts": out6[1:5], "reconstruction_error": out6[5], "node_index": idx,
+              "X_mean": Xm.index_select(0, sel).cpu().numpy(), "X_cov": Xc.index_select(0, sel).cpu().numpy()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args, shape):
     import torch
     import torch.distributed as dist
@@ -413,6 +434,10 @@ def run_ours(args, shape):
     e1.record()
     barrier()
     wall1 = time.time()
+    if args.dump_outputs:
+        _lib.check(lib.tame_gather_state(h))      # N > 1: covariance rows from their owners (nothing to do on one GPU)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, Xm, Xc, out6)
     probes = (C.c_uint64 * 16)()
     lib.tame_debug_probes(h, probes)
     probes = list(probes)
@@ -763,7 +788,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (profiling runs)")
     ap.add_argument("--no-extra", action="store_true", help="skip the config-3 / config-5 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     shape = parse_shape(args.config)
     if args.impl == "reference":
         run_reference(args, shape)

@@ -26,7 +26,13 @@ def load_golden(name):
     if not os.path.exists(path):
         pytest.skip(f"golden fixture {name}.npz not generated")
     z = np.load(path)
-    return {k: z[k] for k in z.files}
+    g = {k: z[k] for k in z.files}
+    if "inputs" in g:           # runs of one problem share its inputs (Y, X_true, initial states) in one fixture
+        g = {**load_golden(str(g.pop("inputs"))), **g}
+    if "Y0" in g:               # mirror-consistent Y stored as its first channel: Y[i, j, t, 1] == Y[j, i, t, 0]
+        Y0 = g.pop("Y0")
+        g["Y"] = np.stack([Y0, np.swapaxes(Y0, 0, 1)], axis=-1)
+    return g
 
 
 def golden_constants(g):
