@@ -19,14 +19,13 @@ sys.path.insert(0, os.path.join(ROOT, "python-temporal-ame-svi_b200")); sys.path
 from tame_b200 import _lib
 from tame_b200.sharding import shard_rows
 from oracle import tame_oracle as orc
-from gpu_util import make_config
-from test_gpu_parity import _random_problem
+from gpu_util import make_config, random_problem
 rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
 torch.cuda.set_device(rank); dev = torch.device("cuda", rank)
 dist.init_process_group("nccl", device_id=dev)
 lib = _lib.load()
 n, T, r, lr, iters = 256, 9, 3, 0.3, 2
-c, Y, Xm, Xc = _random_problem(n, T, r, seed=77)
+c, Y, Xm, Xc = random_problem(n, T, r, seed=77)
 if os.environ.get("TAME_TEST_ASYM") == "1":
     Y = Y.copy(); Y[3, 200, 2, 0] += 0.125          # one dyad no longer mirror-consistent -> full ELBO pass on every rank
 for meth in ("good", "naive"):

@@ -5,13 +5,10 @@ import pytest
 import torch
 
 from conftest import GOLDEN_CASES, GOLDEN_LONG, METHODS, golden_constants, load_golden, rel_err
+from gpu_util import TOL, UNSTABLE, random_problem, trace_ok
 from oracle import tame_oracle as orc
 
 pytestmark = pytest.mark.gpu
-TOL = 1e-9
-# divergent iterations in the reference itself ('bad' with a large step): rounding differences are amplified
-# each sweep, so the comparison window is the first iterations and the tolerance widens with the sweep count.
-UNSTABLE = {("conftest_lr1", "bad"), ("r3_rho08", "bad"), ("r1_T1", "bad"), ("r4_T2", "bad")}
 
 
 @pytest.fixture(autouse=True)
@@ -20,11 +17,6 @@ def _float64_default():
     torch.set_default_dtype(torch.float64)
     yield
     torch.set_default_dtype(old)
-
-
-def _trace_ok(a, b, tol=TOL):
-    a, b = np.asarray(a), np.asarray(b)
-    return a.shape == b.shape and np.all(np.abs(a - b) <= tol * np.abs(b))
 
 
 @pytest.mark.parametrize("meth", METHODS)
@@ -39,10 +31,10 @@ def test_c_abi_fit_matches_reference_golden(case, meth):
     ref_el, ref_ms = g[f"{meth}_elbo"], g[f"{meth}_mse"]
     assert len(el) == len(ref_el), "early-stop iteration differs"
     if (case, meth) in UNSTABLE:
-        assert _trace_ok(el[:2], ref_el[:2], 1e-8) and _trace_ok(ms[:2], ref_ms[:2], 1e-8)
+        assert trace_ok(el[:2], ref_el[:2], 1e-8) and trace_ok(ms[:2], ref_ms[:2], 1e-8)
         return
-    assert _trace_ok(el, ref_el), np.max(np.abs(el - ref_el) / np.abs(ref_el))
-    assert _trace_ok(ms, ref_ms), np.max(np.abs(ms - ref_ms) / np.abs(ref_ms))
+    assert trace_ok(el, ref_el), np.max(np.abs(el - ref_el) / np.abs(ref_el))
+    assert trace_ok(ms, ref_ms), np.max(np.abs(ms - ref_ms) / np.abs(ref_ms))
     assert rel_err(Xm, g[f"{meth}_final_mean"]) < TOL
     assert rel_err(Xc, g[f"{meth}_final_cov"]) < TOL
 
@@ -62,38 +54,17 @@ def test_drop_in_classes_match_reference_golden(case, meth):
     iters = min(int(g["max_iter"]), 25)
     hist = vi.fit(max_iter=iters, tolerance=0.0, verbose=False)
     assert hist is vi.history and len(hist["elbo"]) == iters
-    assert _trace_ok(hist["elbo"], g[f"{meth}_elbo"][:iters])
-    assert _trace_ok(hist["reconstruction_error"], g[f"{meth}_mse"][:iters])
+    assert trace_ok(hist["elbo"], g[f"{meth}_elbo"][:iters])
+    assert trace_ok(hist["reconstruction_error"], g[f"{meth}_mse"][:iters])
     if iters == int(g["max_iter"]):
         assert rel_err(vi.get_variational_means().numpy(), g[f"{meth}_final_mean"]) < TOL
         assert rel_err(vi.get_variational_covariances().numpy(), g[f"{meth}_final_cov"]) < TOL
         parts = [vi._compute_expected_log_likelihood(), vi._compute_log_prior_initial(),
                  vi._compute_log_prior_transitions(), vi._compute_entropy()]
-        assert _trace_ok(parts, g[f"{meth}_parts"])
+        assert trace_ok(parts, g[f"{meth}_parts"])
     # a second fit() continues from the current state and appends to the same history (base.py:176-180)
     vi.fit(max_iter=2, tolerance=0.0, verbose=False)
     assert len(vi.history["elbo"]) == iters + 2
-
-
-def _random_problem(n, T, r, seed, rho=0.5, ar=0.8):
-    rng = np.random.default_rng(seed)
-    c = orc.model_constants(n, T, r, ar_coefficient=ar, rho_dyadic=rho)
-    d = c["d"]
-    X = rng.standard_normal((n, T, d)) * 0.7
-    Y = np.zeros((n, n, T, 2))
-    Lr = np.linalg.cholesky(c["R"])
-    for t in range(T):
-        mu = orc.compute_mean(X[:, t, :2], X[:, t, 2:], r)
-        eps = rng.standard_normal((n, n, 2)) @ Lr.T
-        yt = mu + eps
-        iu = np.triu_indices(n, 1)
-        Y[iu[0], iu[1], t] = yt[iu]
-        Y[iu[1], iu[0], t, 0] = yt[iu][:, 1]
-        Y[iu[1], iu[0], t, 1] = yt[iu][:, 0]
-    Xm = rng.standard_normal((n, T, d)) * 0.1
-    G = rng.standard_normal((n, T, d, d)) * 0.01
-    Xc = 0.6 * np.eye(d) + 0.5 * (G + np.swapaxes(G, -1, -2))
-    return c, Y, Xm, Xc
 
 
 # shapes that cross the 64-node block boundary (upper pass, pushes, several chain launches), ragged n and T,
@@ -120,7 +91,7 @@ def sweep_path(request, monkeypatch):
 def test_c_abi_matches_oracle_on_seeded_inputs(shape, meth, sweep_path):
     from gpu_util import fit_host
     n, T, r = shape
-    c, Y, Xm, Xc = _random_problem(n, T, r, seed=1000 + n + T + r, rho=0.5 if r % 2 else -0.3)
+    c, Y, Xm, Xc = random_problem(n, T, r, seed=1000 + n + T + r, rho=0.5 if r % 2 else -0.3)
     lr = 0.05 if meth == "bad" else 0.3
     mode = orc.MODE_OF[meth]
     iters = 2
@@ -133,7 +104,7 @@ def test_c_abi_matches_oracle_on_seeded_inputs(shape, meth, sweep_path):
         oms.append(orc.reconstruction_mse(Y, Om, c))
     assert rel_err(Gm, Om) < TOL, rel_err(Gm, Om)
     assert rel_err(Gc, Oc) < TOL, rel_err(Gc, Oc)
-    assert _trace_ok(el, oel) and _trace_ok(ms, oms)
+    assert trace_ok(el, oel) and trace_ok(ms, oms)
 
 
 def test_asymmetric_Y_and_general_dynamics():
@@ -142,7 +113,7 @@ def test_asymmetric_Y_and_general_dynamics():
     from gpu_util import fit_host
     rng = np.random.default_rng(7)
     n, T, r = 80, 6, 2
-    c, Y, Xm, Xc = _random_problem(n, T, r, seed=5)
+    c, Y, Xm, Xc = random_problem(n, T, r, seed=5)
     Y = Y + rng.standard_normal(Y.shape) * 0.3
     Y[np.arange(n), np.arange(n)] = rng.standard_normal((n, T, 2))     # diagonal must be ignored
     d = c["d"]
@@ -165,7 +136,7 @@ def test_handle_level_calls_and_properties():
     'bad' keeps its cross blocks at zero; naive covariances stay diagonal (test_inference.py:187-203, 37-43)."""
     from gpu_util import DeviceFit
     n, T, r = 90, 5, 2
-    c, Y, Xm, Xc = _random_problem(n, T, r, seed=11)
+    c, Y, Xm, Xc = random_problem(n, T, r, seed=11)
     f = DeviceFit(Y, Xm, Xc, c, 0.0, orc.GOOD)
     before = f.elbo_mse()
     f.sweep()
@@ -242,10 +213,7 @@ def test_fit_batch_matches_per_fit_oracle(path, monkeypatch):
     """BASELINE config 5 in miniature: a grid of independent small fits (n, T, r, ar, rho vary; all three methods) through
     tame_fit_batch, each compared with the oracle's fit() including the per-fit early stop.  Default path: one launch of the
     whole-fit kernel per fit (k_fit, both team shapes); TAME_BATCH=host: the host-driven loop."""
-    import ctypes as C
-    from gpu_util import make_config
-    from tame_b200 import _lib
-    lib = _lib.load()
+    from gpu_util import run_batch
     monkeypatch.delenv("TAME_BATCH", raising=False)
     monkeypatch.delenv("TAME_NH", raising=False)
     if path == "host-loop":
@@ -254,34 +222,25 @@ def test_fit_batch_matches_per_fit_oracle(path, monkeypatch):
         monkeypatch.setenv("TAME_NH", "1")
     grid = [(10, 5, 0.8, 0.5, 2), (24, 8, 0.5, 0.0, 2), (40, 3, 0.9, 0.8, 2), (33, 12, 0.3, -0.3, 2), (70, 4, 0.8, 0.5, 2),
             (12, 20, 0.7, 0.2, 2), (130, 7, 0.8, 0.5, 8), (96, 33, 0.6, 0.3, 3)]
-    fits, keep = [], []
+    fits = []
     for k, (n, T, ar, rho, r) in enumerate(grid):
         for meth in (("naive", "good") if r == 2 else ("good", "bad")):
-            c, Y, Xm, Xc = _random_problem(n, T, r, seed=300 + k, rho=rho, ar=ar)
-            fits.append((c, Y, Xm, Xc, meth))
-    nf, max_iter, tol = len(fits), 12, 2e-2
-    cfgs = (_lib.TameConfig * nf)()
-    Yp, Mp, Cp = (C.c_void_p * nf)(), (C.c_void_p * nf)(), (C.c_void_p * nf)()
-    dev = []
-    lr_of = lambda meth: 0.05 if meth == "bad" else 0.3
-    for f, (c, Y, Xm, Xc, meth) in enumerate(fits):
-        cfg, kk = make_config(c, lr_of(meth), orc.MODE_OF[meth])
-        keep.append(kk)
-        cfgs[f] = cfg
-        t = [torch.as_tensor(a, dtype=torch.float64).cuda().contiguous() for a in (Y, Xm, Xc)]
-        dev.append(t)
-        Yp[f], Mp[f], Cp[f] = t[0].data_ptr(), t[1].data_ptr(), t[2].data_ptr()
-    torch.cuda.synchronize()
-    el = np.zeros((nf, max_iter)); ms = np.zeros((nf, max_iter)); nd = (C.c_int32 * nf)()
-    _lib.check(lib.tame_fit_batch(nf, cfgs, Yp, Mp, Cp, max_iter, tol, _lib.dptr(el), _lib.dptr(ms), nd, 4))
+            c, Y, Xm, Xc = random_problem(n, T, r, seed=300 + k, rho=rho, ar=ar)
+            fits.append((c, Y, Xm, Xc, 0.05 if meth == "bad" else 0.3, orc.MODE_OF[meth]))
+    max_iter, tol = 12, 2e-2
+    traces, n_done, states, launches = run_batch(fits, max_iter, tol, n_streams=4)
+    if path == "host-loop":
+        assert launches > 2 * len(fits)
+    else:
+        assert launches == 2 * len(fits), "one k_hab and one k_fit per fit"
     stopped_early = 0
-    for f, (c, Y, Xm, Xc, meth) in enumerate(fits):
+    for f, (c, Y, Xm, Xc, lr, mode) in enumerate(fits):
         Om, Oc = Xm.copy(), Xc.copy()
-        oel, oms = orc.fit(Y, Om, Oc, c, lr_of(meth), orc.MODE_OF[meth], max_iter, tol, blocked=(c["n"] > 80))
-        assert nd[f] == len(oel), (f, nd[f], len(oel))
+        oel, oms = orc.fit(Y, Om, Oc, c, lr, mode, max_iter, tol, blocked=(c["n"] > 80))
+        assert n_done[f] == len(oel), (f, n_done[f], len(oel))
         stopped_early += len(oel) < max_iter
-        assert _trace_ok(el[f, :nd[f]], oel) and _trace_ok(ms[f, :nd[f]], oms)
-        assert rel_err(dev[f][1].cpu().numpy(), Om) < TOL and rel_err(dev[f][2].cpu().numpy(), Oc) < TOL
+        assert trace_ok(traces[f][0], oel) and trace_ok(traces[f][1], oms)
+        assert rel_err(states[f][0], Om) < TOL and rel_err(states[f][1], Oc) < TOL
     assert stopped_early > 0, "the test should exercise the per-fit early stop"
 
 
@@ -293,7 +252,7 @@ def test_elbo_pass_variants_agree_with_oracle(shape, variant, monkeypatch):
     from gpu_util import DeviceFit
     monkeypatch.setenv("TAME_LLMSE", variant)
     n, T, r = shape
-    c, Y, Xm, Xc = _random_problem(n, T, r, seed=4242 + n)
+    c, Y, Xm, Xc = random_problem(n, T, r, seed=4242 + n)
     for asym in (False, True):
         Yt = Y.copy()
         if asym:
@@ -314,7 +273,7 @@ def test_hundred_sweeps_no_drift(meth, sweep_path):
     schedule: whole ELBO / MSE traces and the final state at rel 1e-9."""
     from gpu_util import fit_host
     n, T, r, iters = 200, 12, 4, 100
-    c, Y, Xm, Xc = _random_problem(n, T, r, seed=77, rho=0.5)
+    c, Y, Xm, Xc = random_problem(n, T, r, seed=77, rho=0.5)
     lr, mode = 0.3, orc.MODE_OF[meth]
     el, ms, Gm, Gc = fit_host(Y, Xm, Xc, c, lr, mode, iters)
     Om, Oc = Xm.copy(), Xc.copy()
@@ -325,7 +284,7 @@ def test_hundred_sweeps_no_drift(meth, sweep_path):
         oms.append(orc.reconstruction_mse(Y, Om, c))
     assert rel_err(Gm, Om) < TOL, rel_err(Gm, Om)
     assert rel_err(Gc, Oc) < TOL, rel_err(Gc, Oc)
-    assert _trace_ok(el, oel) and _trace_ok(ms, oms)
+    assert trace_ok(el, oel) and trace_ok(ms, oms)
 
 
 def test_deterministic_mode_is_bitwise_reproducible(monkeypatch):
@@ -333,7 +292,7 @@ def test_deterministic_mode_is_bitwise_reproducible(monkeypatch):
     same fit give bit-identical traces and state (the default order depends on timing at the 1e-16 level)."""
     from gpu_util import fit_host
     monkeypatch.setenv("TAME_DETERMINISTIC", "1")
-    c, Y, Xm, Xc = _random_problem(700, 5, 2, seed=5, rho=0.4)
+    c, Y, Xm, Xc = random_problem(700, 5, 2, seed=5, rho=0.4)
     a = fit_host(Y, Xm, Xc, c, 0.3, orc.GOOD, 3)
     b = fit_host(Y, Xm, Xc, c, 0.3, orc.GOOD, 3)
     assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
