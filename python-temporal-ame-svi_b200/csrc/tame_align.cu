@@ -10,6 +10,7 @@
 //   k_align_apply   rotate the U / V rows, per-row sign flips of the (a,b), U and V parts, squared error
 //   k_align_sum     fixed-order reduction of the partial sums
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 #include <cmath>
 #include <cstdint>
@@ -560,11 +561,15 @@ __global__ void k_diag_contrib(const double* __restrict__ sums, const double* __
         mul -= q[5];
         cnt = nn * (nn - 1.0);
     }
-    additive[t] = add / cnt;
-    multiplicative[t] = mul / cnt;
+    // n = 1 without the diagonal has no pair: the mean over none is NaN (add and mul are rounding residues there)
+    additive[t] = cnt > 0.0 ? add / cnt : CUDART_NAN;
+    multiplicative[t] = cnt > 0.0 ? mul / cnt : CUDART_NAN;
 }
 
 // Pearson correlation of the flattened n x n products U V' (diagonal included), one thread per time step.
+// When either side's products are all zero (its U or V block is zero) the variance is exactly 0 and the correlation is
+// undefined: NaN, as torch.corrcoef returns.  A variance <= 0 from rounding is treated the same, and the clamp to [-1, 1]
+// passes NaN through (fmax(-1, NaN) would return -1).
 __global__ void k_diag_corr(const double* __restrict__ sums_e, const double* __restrict__ sums_t, const double* __restrict__ gram_e,
                             const double* __restrict__ gram_t, const double* __restrict__ cross, int n, int T, int r,
                             double* __restrict__ corr) {
@@ -591,8 +596,12 @@ __global__ void k_diag_corr(const double* __restrict__ sums_e, const double* __r
     double c = 0.0;
     if (N > 1.0) {                                   // multiplicative_strength_comparison.py:82-86
         const double cov = ste - st * se / N, ve = see - se * se / N, vt = stt - st * st / N;
-        c = cov / sqrt(ve * vt);
-        c = fmin(1.0, fmax(-1.0, c));                // torch.corrcoef clips to [-1, 1]
+        if (ve > 0.0 && vt > 0.0) {
+            c = cov / sqrt(ve * vt);
+            c = c > 1.0 ? 1.0 : (c < -1.0 ? -1.0 : c);     // torch.corrcoef clips to [-1, 1]; NaN stays NaN
+        } else {
+            c = CUDART_NAN;
+        }
     }
     corr[t] = c;
 }

@@ -3,7 +3,9 @@ compute_uv_correlation_over_time of experiments/multiplicative_strength_comparis
 
 Same names, arguments and return types as the reference.  The reference materialises the n x n matrices a_i + b_j and
 U_i.V_j per time step; libtame_b200 (csrc/tame_align.cu) gets the same sums from r x r Gram matrices computed on the
-FP64 tensor cores plus per-time-step row sums -- O(n T r^2) instead of O(n^2 T r).  No CPU implementation: without the CUDA
+FP64 tensor cores plus per-time-step row sums -- O(n T r^2) instead of O(n^2 T r).  Undefined values are NaN, as in the
+reference: the U'V correlation of a time step where either side's products are all zero (a zero U or V block), and
+contributions over no pair (n = 1 with exclude_diagonal).  No CPU implementation: without the CUDA
 library these functions raise.  The printing / bookkeeping helpers of the reference module (print_diagnostic_summary,
 compare_methods, track_convergence, compute_elbo_gap, compute_reconstruction_error) are host-side utilities outside
 the accelerated path and are not provided.
