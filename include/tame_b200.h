@@ -89,6 +89,11 @@ int tame_local_rows(const tame_handle* h, int32_t* n_rows_local);
  * pass that builds the sweep-invariant sums  h_a[i,t] = sum_{j!=i} (p*y0 + q*y1),  h_b[i,t] = sum (q*y0 + p*y1)
  * -- the [a,b] rows of sum_j J'R^-1 y_ij in structured_mf.py:324.                                            */
 int tame_bind_Y(tame_handle* h, const double* Y_dev);
+/* The same for float observations (the reference's default dtype): Y stays float in HBM, half the bytes of the
+ * double layout, and every dyad is widened to double when a kernel loads it -- the arithmetic, the state and the
+ * results are those of tame_bind_Y on the widened Y, bit for bit.  The handle remembers the element type until the
+ * next bind; rebinding with the other type is allowed. */
+int tame_bind_Y_f32(tame_handle* h, const float* Y_dev);
 /* Bind the variational state; it is updated IN PLACE like the reference's self.X_mean / self.X_cov
  * (structured_mf.py:282-287). */
 int tame_bind_state(tame_handle* h, double* X_mean_dev, double* X_cov_dev);
@@ -120,6 +125,10 @@ int tame_fit_device(tame_handle* h, int32_t max_iter, double tolerance, double* 
 int tame_fit_host(const tame_config* cfg, const double* Y_host, double* X_mean_host, double* X_cov_host,
                   int32_t max_iter, double tolerance, double* elbo_trace_host, double* mse_trace_host,
                   int32_t* n_done);
+/* tame_fit_host with float Y (tame_bind_Y_f32): stages half the bytes of Y; the state stays double. */
+int tame_fit_host_f32(const tame_config* cfg, const float* Y_host, double* X_mean_host, double* X_cov_host,
+                      int32_t max_iter, double tolerance, double* elbo_trace_host, double* mse_trace_host,
+                      int32_t* n_done);
 
 /* BASELINE config 5 (experiments/sensitivity_analysis.py:117-183: many independent small fits, one per grid point
  * and method): n_fits independent problems, each with its own tame_config and device buffers (Y_dev[f] is (n,n,T,2),
@@ -134,6 +143,10 @@ int tame_fit_host(const tame_config* cfg, const double* Y_host, double* X_mean_h
 int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const* Y_dev, double* const* X_mean_dev,
                    double* const* X_cov_dev, int32_t max_iter, double tolerance, double* elbo_traces_host,
                    double* mse_traces_host, int32_t* n_done, int32_t n_streams);
+/* tame_fit_batch with float Y for every fit (tame_bind_Y_f32); everything else as above. */
+int tame_fit_batch_f32(int32_t n_fits, const tame_config* cfgs, const float* const* Y_dev, double* const* X_mean_dev,
+                       double* const* X_cov_dev, int32_t max_iter, double tolerance, double* elbo_traces_host,
+                       double* mse_traces_host, int32_t* n_done, int32_t n_streams);
 
 /* ---- data generation (the step before the path: TemporalAMEModel.generate_data, temporal_ame.py:200-216) - */
 /* Y[i,j,t,:] = (mu0[i,j] + e0, mu0[j,i] + e1), (e0,e1) ~ N(0, R) per unordered dyad and time, mirrored for
@@ -143,6 +156,10 @@ int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const*
  * (row-major, row_end-row_begin rows). */
 int tame_generate_Y(int32_t n, int32_t T, int32_t r, const double R[4], const double* X_true_dev, uint64_t seed,
                     int32_t row_begin, int32_t row_end, double* Y_dev, void* cuda_stream);
+/* The same Y stored as float: computed in double exactly as above and rounded once per value, so it equals
+ * tame_generate_Y's output cast to float and stays mirror-consistent. */
+int tame_generate_Y_f32(int32_t n, int32_t T, int32_t r, const double R[4], const double* X_true_dev, uint64_t seed,
+                        int32_t row_begin, int32_t row_end, float* Y_dev, void* cuda_stream);
 
 /* ---- alignment (the step after the fit in every driver: src/utils/alignment.py; demo.py:135-137) ------------ */
 /* align_temporal_states (alignment.py:224-313) fused with the error of compute_alignment_error (:316-385).

@@ -15,6 +15,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/tame_b200.h"
@@ -112,6 +113,8 @@ struct tame_handle {
     TameParams P{};
     cudaStream_t stream = nullptr;
     bool y_bound = false, state_bound = false, y_symmetric = false;
+    bool y_f32 = false;                  // the bound Y is float (tame_bind_Y_f32): its kernels come from ops->f32
+    const TameYOps& yops() const { return y_f32 ? ops->f32 : ops->f64; }
     bool skip_symcheck = false;          // tame_fit_batch's device-loop path: bind without the mirror check (and its sync)
     double* fit_scratch = nullptr;       // k_fit: per-block partial sums, control block, barrier counter
     int* sym_flag = nullptr;
@@ -179,19 +182,20 @@ static void ev_fold(tame_handle* h) {
 // k_hab: sweep-invariant sums over partners, one pass over Y at bind time.
 //   hab[i,t,0] = sum_{j!=i} p0*y0 + q*y1 ; hab[i,t,1] = sum_{j!=i} q*y0 + p1*y1   (structured_mf.py:324, rows a,b)
 // grid (ceil(T/32), nloc), block (32, 8)
+template <class YT>
 __global__ void __launch_bounds__(256) k_hab(TameParams P) {
     const int lrow = blockIdx.y;
     const int i = tame_grow(lrow, P.panel, P.world, P.rank);
     const int t = blockIdx.x * 32 + threadIdx.x;
     const bool tv = t < P.T;
     double a0 = 0.0, a1 = 0.0;
-    const double* base = P.Y + ((size_t)lrow * P.n * P.T + (tv ? t : 0)) * 2;
+    const YT* base = TameY<YT>::ptr(P) + ((size_t)lrow * P.n * P.T + (tv ? t : 0)) * 2;
     const size_t jstride = (size_t)P.T * 2;
     int j = threadIdx.y;
     for (; j + 24 < P.n; j += 32) {
         double2 y[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) y[u] = tv ? tame_ld_stream2(base + (size_t)(j + 8 * u) * jstride) : make_double2(0, 0);
+        for (int u = 0; u < 4; ++u) y[u] = tv ? TameY<YT>::wide(TameY<YT>::ld_stream(base + (size_t)(j + 8 * u) * jstride)) : make_double2(0, 0);
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             if (j + 8 * u != i) {
@@ -202,7 +206,7 @@ __global__ void __launch_bounds__(256) k_hab(TameParams P) {
     }
     for (; j < P.n; j += 8) {
         if (tv && j != i) {
-            double2 y = tame_ld_stream2(base + (size_t)j * jstride);
+            double2 y = TameY<YT>::wide(TameY<YT>::ld_stream(base + (size_t)j * jstride));
             a0 += P.p0 * y.x + P.q * y.y;
             a1 += P.q * y.x + P.p1 * y.y;
         }
@@ -226,15 +230,17 @@ __global__ void __launch_bounds__(256) k_hab(TameParams P) {
 // Mirror check at bind time: Y[j,i,t,:] == swap(Y[i,j,t,:]) bit for bit for every i<j (the reference's generate_data
 // writes both entries from one sample, temporal_ame.py:209-216; experiments may overwrite model.Y by hand).  Single GPU
 // only (a rank holds only its own rows).  grid (ceil(T/32), n), block (32, 8); *flag is set to 1 on the first mismatch.
+// Float Y is compared bit for bit as float.
+template <class YT>
 __global__ void __launch_bounds__(256) k_symcheck(TameParams P, int* flag) {
     const int i = blockIdx.y;
     const int t = blockIdx.x * 32 + threadIdx.x;
     if (t >= P.T) return;
     bool bad = false;
     for (int j = i + 1 + threadIdx.y; j < P.n; j += 8) {
-        const double2 a = tame_ld_stream2(P.Y + (((size_t)i * P.n + j) * P.T + t) * 2);
-        const double2 b = tame_ld_stream2(P.Y + (((size_t)j * P.n + i) * P.T + t) * 2);
-        bad |= (__double_as_longlong(a.x) != __double_as_longlong(b.y)) || (__double_as_longlong(a.y) != __double_as_longlong(b.x));
+        const auto a = TameY<YT>::ld_stream(TameY<YT>::ptr(P) + (((size_t)i * P.n + j) * P.T + t) * 2);
+        const auto b = TameY<YT>::ld_stream(TameY<YT>::ptr(P) + (((size_t)j * P.n + i) * P.T + t) * 2);
+        bad |= (TameY<YT>::bits(a.x) != TameY<YT>::bits(b.y)) || (TameY<YT>::bits(a.y) != TameY<YT>::bits(b.x));
     }
     if (bad) *flag = 1;
 }
@@ -247,6 +253,7 @@ __device__ __forceinline__ unsigned long long tame_mix64(unsigned long long x) {
     x ^= x >> 30; x *= 0xbf58476d1ce4e5b9ull; x ^= x >> 27; x *= 0x94d049bb133111ebull; x ^= x >> 31;
     return x;
 }
+template <class YT>
 __global__ void __launch_bounds__(256) k_symhash(TameParams P, unsigned long long* acc) {
     const int lrow = blockIdx.y;
     const int i = tame_grow(lrow, P.panel, P.world, P.rank);
@@ -255,11 +262,11 @@ __global__ void __launch_bounds__(256) k_symhash(TameParams P, unsigned long lon
     if (t < P.T) {
         for (int j = threadIdx.y; j < P.n; j += 8) {
             if (j == i) continue;
-            const double2 y = tame_ld_stream2(P.Y + (((size_t)lrow * P.n + j) * P.T + t) * 2);
+            const auto y = TameY<YT>::ld_stream(TameY<YT>::ptr(P) + (((size_t)lrow * P.n + j) * P.T + t) * 2);
             const int lo = min(i, j), hi = max(i, j);
             const unsigned long long key = ((unsigned long long)lo * P.n + hi) * (unsigned long long)P.T + t;
-            const unsigned long long a = (unsigned long long)__double_as_longlong(i < j ? y.x : y.y);   // y_{lo,hi}
-            const unsigned long long b = (unsigned long long)__double_as_longlong(i < j ? y.y : y.x);   // y_{hi,lo}
+            const unsigned long long a = TameY<YT>::bits(i < j ? y.x : y.y);   // y_{lo,hi}
+            const unsigned long long b = TameY<YT>::bits(i < j ? y.y : y.x);   // y_{hi,lo}
             const unsigned long long h = tame_mix64(tame_mix64(key ^ 0x9e3779b97f4a7c15ull) ^ tame_mix64(a) ^ (tame_mix64(b) * 3ull));
             sum += (i < j) ? h : (0ull - h);
         }
@@ -313,10 +320,12 @@ __global__ void k_finalize(const double* red6, int n, int T, int d, int mode, do
     out6[5] = red6[0] / ((double)n * (double)(n - 1) * (double)T);
 }
 
-// Y generator, one thread per (local row, partner, time).  temporal_ame.py:200-216 in distribution.
+// Y generator, one thread per (local row, partner, time).  temporal_ame.py:200-216 in distribution.  FP64 throughout; a
+// float Y gets each value rounded once when it is stored (both halves of a dyad round the same double: mirror-consistent).
+template <class YT>
 __global__ void __launch_bounds__(256) k_generate(int n, int T, int r, double l00, double l10, double l11,
                                                   const double* __restrict__ X, unsigned long long seed, int row_begin,
-                                                  int row_end, double* __restrict__ Y) {
+                                                  int row_end, YT* __restrict__ Y) {
     const int D = 2 + 2 * r;
     const size_t total = (size_t)(row_end - row_begin) * n * T;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
@@ -341,8 +350,8 @@ __global__ void __launch_bounds__(256) k_generate(int n, int T, int r, double l0
             y0 = mu_ij + (i < j ? e0 : e1);
             y1 = mu_ji + (i < j ? e1 : e0);
         }
-        Y[idx * 2 + 0] = y0;
-        Y[idx * 2 + 1] = y1;
+        Y[idx * 2 + 0] = (YT)y0;
+        Y[idx * 2 + 1] = (YT)y1;
     }
 }
 
@@ -400,7 +409,7 @@ static int tame_reconfigure(tame_handle* h, const tame_config* cfg) {
         h->P.probe_t = T - 1;
         if (const char* v = getenv("TAME_PROBE_T")) h->P.probe_t = std::max(0, std::min(T - 1, atoi(v)));
         const char* v = getenv("TAME_SWEEP");
-        h->fused = !(v && strcmp(v, "panel") == 0) && (T + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 <= h->ops->sweep_capacity(1);
+        h->fused = !(v && strcmp(v, "panel") == 0) && (T + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 <= h->ops->f64.sweep_capacity(1);
         h->nb_ll = h->ops->llmse_blocks(h->P);
         h->nb_cell = h->ops->cellterms_blocks(h->P);
     }
@@ -414,6 +423,64 @@ static int tame_reconfigure(tame_handle* h, const tame_config* cfg) {
     P.p0 = cfg->Rinv[0]; P.p1 = cfg->Rinv[3]; P.q = 0.5 * (cfg->Rinv[1] + cfg->Rinv[2]);
     P.Y = nullptr; P.Xm = nullptr; P.Xc = nullptr;
     h->y_bound = h->state_bound = h->y_symmetric = false;
+    return TAME_OK;
+}
+
+// tame_bind_Y / tame_bind_Y_f32: the handle remembers the element type, every later launch takes that type's kernels
+template <class YT>
+static int bind_Y(tame_handle* h, const YT* Y) {
+    if (!h || !Y) return fail(TAME_EINVAL, "null argument");
+    CK(cudaSetDevice(h->cfg.device));
+    h->P.Y = Y;
+    h->y_f32 = std::is_same<YT, float>::value;
+    dim3 grid((h->P.T + 31) / 32, h->nloc), block(32, 8);
+    k_hab<YT><<<grid, block, 0, h->stream>>>(h->P);
+    tame_count_launch(1);
+    CK(cudaGetLastError());
+    // mirror property of Y (single GPU): lets the ELBO/MSE pass stream only the i<j half.  TAME_SYMMETRIC=0 disables.
+    h->y_symmetric = false;
+    const char* sv = getenv("TAME_SYMMETRIC");
+    if (h->skip_symcheck) { h->y_bound = true; return TAME_OK; }
+    if (h->P.world == 1 && !(sv && atoi(sv) == 0)) {
+        CK(cudaMemsetAsync(h->sym_flag, 0, sizeof(int), h->stream));
+        k_symcheck<YT><<<grid, block, 0, h->stream>>>(h->P, h->sym_flag);
+        tame_count_launch(1);
+        int bad = 1;
+        CK(cudaMemcpyAsync(&bad, h->sym_flag, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        h->y_symmetric = (bad == 0);
+    }
+    if (h->P.world > 1 && h->comm && !(sv && atoi(sv) == 0)) {
+        // multi-GPU: signed hash sum over every rank's rows (needs tame_comm_init before tame_bind_Y)
+        unsigned long long* acc = nullptr;
+        CK(cudaMalloc((void**)&acc, sizeof(unsigned long long)));
+        CK(cudaMemsetAsync(acc, 0, sizeof(unsigned long long), h->stream));
+        k_symhash<YT><<<grid, block, 0, h->stream>>>(h->P, acc);
+        tame_count_launch(1);
+        NK(g_nccl.AllReduce(acc, acc, 1, ncclUint64, ncclSum, h->comm, h->stream));
+        unsigned long long total = 1;
+        CK(cudaMemcpyAsync(&total, acc, sizeof(total), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        cudaFree(acc);
+        h->y_symmetric = (total == 0ull);
+    }
+    h->y_bound = true;
+    return TAME_OK;
+}
+
+template <class YT>
+static int generate_Y(int32_t n, int32_t T, int32_t r, const double R[4], const double* X_dev, uint64_t seed,
+                      int32_t row_begin, int32_t row_end, YT* Y_dev, void* stream) {
+    if (!R || !X_dev || !Y_dev || row_begin < 0 || row_end > n || row_end < row_begin) return fail(TAME_EINVAL, "bad argument");
+    if (R[0] <= 0) return fail(TAME_EINVAL, "R must be positive definite");
+    const double l00 = std::sqrt(R[0]), l10 = R[2] / l00, l11sq = R[3] - l10 * l10;
+    if (l11sq <= 0) return fail(TAME_EINVAL, "R must be positive definite");
+    const size_t total = (size_t)(row_end - row_begin) * n * T;
+    if (total == 0) return TAME_OK;
+    const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 64);
+    k_generate<YT><<<blocks, 256, 0, (cudaStream_t)stream>>>(n, T, r, l00, l10, std::sqrt(l11sq), X_dev, seed, row_begin, row_end, Y_dev);
+    tame_count_launch(1);
+    CK(cudaGetLastError());
     return TAME_OK;
 }
 
@@ -496,7 +563,9 @@ int tame_create(const tame_config* cfg, tame_handle** out) {
         const char* v = getenv("TAME_SWEEP");   // "panel" forces the stream-ordered per-panel path (debug / comparison)
         h->fused = (world == 1) && !(v && strcmp(v, "panel") == 0);
         h->fused_multi = !(v && strcmp(v, "panel") == 0);
-        if (h->fused && (T + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 > h->ops->sweep_capacity(1)) h->fused = false;
+        // the element type of Y is not known yet: the double instantiation is the binding one (the float one has the same
+        // launch bounds and a smaller shared-memory footprint, so at least its capacity)
+        if (h->fused && (T + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 > h->ops->f64.sweep_capacity(1)) h->fused = false;
     }
 
     TameParams& P = h->P;
@@ -554,44 +623,8 @@ int tame_local_rows(const tame_handle* h, int32_t* out) {
     return TAME_OK;
 }
 
-int tame_bind_Y(tame_handle* h, const double* Y) {
-    if (!h || !Y) return fail(TAME_EINVAL, "null argument");
-    CK(cudaSetDevice(h->cfg.device));
-    h->P.Y = Y;
-    dim3 grid((h->P.T + 31) / 32, h->nloc), block(32, 8);
-    k_hab<<<grid, block, 0, h->stream>>>(h->P);
-    tame_count_launch(1);
-    CK(cudaGetLastError());
-    // mirror property of Y (single GPU): lets the ELBO/MSE pass stream only the i<j half.  TAME_SYMMETRIC=0 disables.
-    h->y_symmetric = false;
-    const char* sv = getenv("TAME_SYMMETRIC");
-    if (h->skip_symcheck) { h->y_bound = true; return TAME_OK; }
-    if (h->P.world == 1 && !(sv && atoi(sv) == 0)) {
-        CK(cudaMemsetAsync(h->sym_flag, 0, sizeof(int), h->stream));
-        k_symcheck<<<grid, block, 0, h->stream>>>(h->P, h->sym_flag);
-        tame_count_launch(1);
-        int bad = 1;
-        CK(cudaMemcpyAsync(&bad, h->sym_flag, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        h->y_symmetric = (bad == 0);
-    }
-    if (h->P.world > 1 && h->comm && !(sv && atoi(sv) == 0)) {
-        // multi-GPU: signed hash sum over every rank's rows (needs tame_comm_init before tame_bind_Y)
-        unsigned long long* acc = nullptr;
-        CK(cudaMalloc((void**)&acc, sizeof(unsigned long long)));
-        CK(cudaMemsetAsync(acc, 0, sizeof(unsigned long long), h->stream));
-        k_symhash<<<grid, block, 0, h->stream>>>(h->P, acc);
-        tame_count_launch(1);
-        NK(g_nccl.AllReduce(acc, acc, 1, ncclUint64, ncclSum, h->comm, h->stream));
-        unsigned long long total = 1;
-        CK(cudaMemcpyAsync(&total, acc, sizeof(total), cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        cudaFree(acc);
-        h->y_symmetric = (total == 0ull);
-    }
-    h->y_bound = true;
-    return TAME_OK;
-}
+int tame_bind_Y(tame_handle* h, const double* Y) { return bind_Y<double>(h, Y); }
+int tame_bind_Y_f32(tame_handle* h, const float* Y) { return bind_Y<float>(h, Y); }
 
 int tame_bind_state(tame_handle* h, double* Xm, double* Xc) {
     if (!h || !Xm || !Xc) return fail(TAME_EINVAL, "null argument");
@@ -617,6 +650,7 @@ int tame_sweep(tame_handle* h) {
     CK(cudaSetDevice(h->cfg.device));
     const TameParams& P = h->P;
     const TameOps* ops = h->ops;
+    const TameYOps& yops = h->yops();
     const int n = P.n, T = P.T, d = h->d, world = P.world, rank = P.rank;
     cudaStream_t st = h->stream;
     ev_mark(h, 0);
@@ -627,19 +661,19 @@ int tame_sweep(tame_handle* h) {
     if (h->fused || (world > 1 && h->npeers == world - 1 && h->fused_multi)) {
         // single GPU: the whole sweep is one persistent cooperative launch (chain CTAs + streaming CTAs)
         ev_mark(h, 2);
-        cudaError_t e = ops->sweep_fused(h->P, st);
+        cudaError_t e = yops.sweep_fused(h->P, st);
         if (e != cudaSuccess) return fail(TAME_ECUDA, "fused sweep launch: %s", cudaGetErrorString(e));
         ev_mark(h, 0);
     } else {
         // static upper part: partners j > k still carry their old means when row k is updated
-        ops->contract(P, 0, n, 0, n, /*tri=*/1, /*accumulate=*/0, st);
+        yops.contract(P, 0, n, 0, n, /*tri=*/1, /*accumulate=*/0, st);
         ev_mark(h, 0);
         for (int lo = 0; lo < n; lo += TAME_WIN) {
             const int hi = std::min(n, lo + TAME_WIN);
             const int owner = (lo / h->panel) % world;
             if (owner == rank) {
                 ev_mark(h, 2);
-                cudaError_t e = ops->chain(P, lo, hi, st);
+                cudaError_t e = yops.chain(P, lo, hi, st);
                 if (e != cudaSuccess) return fail(TAME_ECUDA, "chain launch: %s", cudaGetErrorString(e));
                 ev_mark(h, 0);
             }
@@ -653,7 +687,7 @@ int tame_sweep(tame_handle* h) {
             if (hi < n) {
                 // right-looking push: the block's new means reach every later row
                 ev_mark(h, 1);
-                ops->contract(P, hi, n, lo, hi, /*tri=*/0, /*accumulate=*/1, st);
+                yops.contract(P, hi, n, lo, hi, /*tri=*/0, /*accumulate=*/1, st);
                 ev_mark(h, 0);
             }
         }
@@ -672,7 +706,7 @@ int tame_elbo_mse(tame_handle* h, double* out6_host) {
     cudaStream_t st = h->stream;
     int nb = 0;
     ev_mark(h, 3);
-    h->ops->llmse(P, h->part_ll, &nb, h->y_symmetric ? 1 : 0, st);
+    h->yops().llmse(P, h->part_ll, &nb, h->y_symmetric ? 1 : 0, st);
     ev_mark(h, 0);
     h->ops->cellterms(P, h->cfg.logdet_S0, h->cfg.logdet_Q, h->part_cell, h->nb_cell, st);
     k_reduce6<<<1, 256, 0, st>>>(h->part_ll, nb, h->part_cell, h->nb_cell, h->red6);
@@ -729,7 +763,7 @@ int tame_fit_device(tame_handle* h, int32_t max_iter, double tolerance, double* 
     if (h->P.world != 1 || !h->fused) return fail(TAME_EINVAL, "tame_fit_device needs the single-GPU fused sweep");
     if (max_iter <= 0) return fail(TAME_EINVAL, "max_iter must be positive");
     CK(cudaSetDevice(h->cfg.device));
-    if (h->ops->fit_grid(h->P) > 1024) return fail(TAME_EINVAL, "problem too large for the whole-fit kernel");
+    if (h->yops().fit_grid(h->P) > 1024) return fail(TAME_EINVAL, "problem too large for the whole-fit kernel");
     cudaStream_t st = h->stream;
     CK(cudaMemsetAsync(h->fit_scratch + FIT_PART_DOUBLES, 0, sizeof(double) * 8, st));      // ctl[0..2], barrier counter
     CK(cudaMemsetAsync(n_done_dev, 0, sizeof(int32_t), st));
@@ -742,17 +776,20 @@ int tame_fit_device(tame_handle* h, int32_t max_iter, double tolerance, double* 
     F.ctl = h->fit_scratch + FIT_PART_DOUBLES;
     F.bar = reinterpret_cast<unsigned int*>(h->fit_scratch + FIT_PART_DOUBLES + 4);
     h->P.epoch = h->epoch;               // iteration `it` of the kernel stamps with epoch + it + 1
-    cudaError_t e = h->ops->fit_device(h->P, F, nullptr, st);
+    cudaError_t e = h->yops().fit_device(h->P, F, nullptr, st);
     h->epoch += max_iter;
     h->P.epoch = h->epoch;
     if (e != cudaSuccess) return fail(TAME_ECUDA, "whole-fit kernel launch: %s", cudaGetErrorString(e));
     return TAME_OK;
 }
 
+}  // extern "C"
+
 static constexpr int BATCH_FALLBACK = 1;      // internal: the device-loop path declined before doing any work
 // tame_fit_batch, device-loop path: every fit is ONE cooperative launch of k_fit (all its iterations and its stop rule on
 // the device), queued round-robin on a few streams from this one host thread; nothing comes back to the host until the end.
-static int fit_batch_device(int32_t n_fits, const tame_config* cfgs, const double* const* Y_dev, double* const* Xm_dev,
+template <class YT>
+static int fit_batch_device(int32_t n_fits, const tame_config* cfgs, const YT* const* Y_dev, double* const* Xm_dev,
                             double* const* Xc_dev, int32_t max_iter, double tolerance, double* elbo_traces, double* mse_traces,
                             int32_t* n_done, int32_t n_streams) {
     if (n_streams <= 0) {
@@ -797,7 +834,7 @@ static int fit_batch_device(int32_t n_fits, const tame_config* cfgs, const doubl
     for (int r = 1; r <= TAME_MAX_R; ++r) {
         if (!cap_n[r]) continue;
         // every fit needs the fused sweep (co-resident chain CTAs for all its time steps); otherwise the host loop takes over
-        if ((cap_T[r] + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 > tame_get_ops(r)->sweep_capacity(1)) { cleanup(); return BATCH_FALLBACK; }
+        if ((cap_T[r] + TAME_CHAIN_WPC - 1) / TAME_CHAIN_WPC + 1 > tame_get_ops(r)->f64.sweep_capacity(1)) { cleanup(); return BATCH_FALLBACK; }
         // a batch of very different shapes (large n x small T next to small n x large T) would make the common capacity
         // much larger than any fit: keep one handle per shape then
         const double d = 2 + 2 * r, bytes = (double)S * cap_n[r] * cap_T[r] * (3.0 * d * d + 8.0 * d) * 8.0;
@@ -818,7 +855,7 @@ static int fit_batch_device(int32_t n_fits, const tame_config* cfgs, const doubl
         }
         if (rc == TAME_OK) rc = tame_reconfigure(h, &cf);
         if (rc == TAME_OK && !h->fused) rc = fail(TAME_ESTATE, "tame_fit_batch: the fused sweep is unavailable for fit %d", f);
-        if (rc == TAME_OK) rc = tame_bind_Y(h, Y_dev[f]);
+        if (rc == TAME_OK) rc = bind_Y<YT>(h, Y_dev[f]);
         if (rc == TAME_OK) rc = tame_bind_state(h, Xm_dev[f], Xc_dev[f]);
         if (rc == TAME_OK) rc = tame_fit_device(h, max_iter, tolerance, el_d + (size_t)f * max_iter, ms_d + (size_t)f * max_iter, nd_d + f);
     }
@@ -845,7 +882,8 @@ static int fit_batch_device(int32_t n_fits, const tame_config* cfgs, const doubl
     return rc;
 }
 
-int tame_fit_host(const tame_config* cfg, const double* Y_host, double* Xm_host, double* Xc_host, int32_t max_iter,
+template <class YT>
+static int fit_host(const tame_config* cfg, const YT* Y_host, double* Xm_host, double* Xc_host, int32_t max_iter,
                   double tolerance, double* elbo_trace, double* mse_trace, int32_t* n_done) {
     if (!cfg || !Y_host || !Xm_host || !Xc_host) return fail(TAME_EINVAL, "null argument");
     if (cfg->world != 1) return fail(TAME_EINVAL, "tame_fit_host is single-GPU");
@@ -853,8 +891,9 @@ int tame_fit_host(const tame_config* cfg, const double* Y_host, double* Xm_host,
     int rc = tame_create(cfg, &h);
     if (rc != TAME_OK) return rc;
     const size_t n = cfg->n, T = cfg->T, d = 2 + 2 * cfg->r;
-    const size_t by = sizeof(double) * n * n * T * 2, bm = sizeof(double) * n * T * d, bc = bm * d;
-    double *Y = nullptr, *Xm = nullptr, *Xc = nullptr;
+    const size_t by = sizeof(YT) * n * n * T * 2, bm = sizeof(double) * n * T * d, bc = bm * d;
+    YT* Y = nullptr;
+    double *Xm = nullptr, *Xc = nullptr;
     cudaError_t e = cudaMalloc((void**)&Y, by);
     if (e == cudaSuccess) e = cudaMalloc((void**)&Xm, bm);
     if (e == cudaSuccess) e = cudaMalloc((void**)&Xc, bc);
@@ -862,7 +901,7 @@ int tame_fit_host(const tame_config* cfg, const double* Y_host, double* Xm_host,
     if (e == cudaSuccess) e = cudaMemcpyAsync(Xm, Xm_host, bm, cudaMemcpyHostToDevice, h->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(Xc, Xc_host, bc, cudaMemcpyHostToDevice, h->stream);
     if (e != cudaSuccess) rc = fail(TAME_ECUDA, "tame_fit_host staging: %s", cudaGetErrorString(e));
-    if (rc == TAME_OK) rc = tame_bind_Y(h, Y);
+    if (rc == TAME_OK) rc = bind_Y<YT>(h, Y);
     if (rc == TAME_OK) rc = tame_bind_state(h, Xm, Xc);
     if (rc == TAME_OK) rc = tame_fit(h, max_iter, tolerance, elbo_trace, mse_trace, n_done);
     if (rc == TAME_OK) {
@@ -878,7 +917,8 @@ int tame_fit_host(const tame_config* cfg, const double* Y_host, double* Xm_host,
     return rc;
 }
 
-int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const* Y_dev, double* const* Xm_dev,
+template <class YT>
+static int fit_batch(int32_t n_fits, const tame_config* cfgs, const YT* const* Y_dev, double* const* Xm_dev,
                    double* const* Xc_dev, int32_t max_iter, double tolerance, double* elbo_traces, double* mse_traces,
                    int32_t* n_done, int32_t n_streams) {
     if (n_fits < 0 || (n_fits > 0 && (!cfgs || !Y_dev || !Xm_dev || !Xc_dev || !n_done))) return fail(TAME_EINVAL, "null argument");
@@ -893,7 +933,7 @@ int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const*
         const char* v = getenv("TAME_BATCH");
         const char* sw = getenv("TAME_SWEEP");
         if (eligible && !(v && strcmp(v, "host") == 0) && !(sw && strcmp(sw, "panel") == 0)) {
-            const int rc = fit_batch_device(n_fits, cfgs, Y_dev, Xm_dev, Xc_dev, max_iter, tolerance, elbo_traces, mse_traces, n_done, n_streams);
+            const int rc = fit_batch_device<YT>(n_fits, cfgs, Y_dev, Xm_dev, Xc_dev, max_iter, tolerance, elbo_traces, mse_traces, n_done, n_streams);
             if (rc != BATCH_FALLBACK) return rc;
         }
     }
@@ -932,7 +972,7 @@ int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const*
                 rc = tame_create(&cf, &h);
                 if (rc == TAME_OK) { pool.push_back(h); rc = tame_set_stream(h, st); }
             }
-            if (rc == TAME_OK) rc = tame_bind_Y(h, Y_dev[f]);
+            if (rc == TAME_OK) rc = bind_Y<YT>(h, Y_dev[f]);
             if (rc == TAME_OK) rc = tame_bind_state(h, Xm_dev[f], Xc_dev[f]);
             if (rc == TAME_OK)
                 rc = tame_fit(h, max_iter, tolerance, elbo_traces ? elbo_traces + (size_t)f * max_iter : nullptr,
@@ -963,19 +1003,35 @@ int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const*
     return TAME_OK;
 }
 
+extern "C" {
+
+int tame_fit_host(const tame_config* cfg, const double* Y_host, double* Xm_host, double* Xc_host, int32_t max_iter,
+                  double tolerance, double* elbo_trace, double* mse_trace, int32_t* n_done) {
+    return fit_host<double>(cfg, Y_host, Xm_host, Xc_host, max_iter, tolerance, elbo_trace, mse_trace, n_done);
+}
+int tame_fit_host_f32(const tame_config* cfg, const float* Y_host, double* Xm_host, double* Xc_host, int32_t max_iter,
+                      double tolerance, double* elbo_trace, double* mse_trace, int32_t* n_done) {
+    return fit_host<float>(cfg, Y_host, Xm_host, Xc_host, max_iter, tolerance, elbo_trace, mse_trace, n_done);
+}
+
+int tame_fit_batch(int32_t n_fits, const tame_config* cfgs, const double* const* Y_dev, double* const* Xm_dev,
+                   double* const* Xc_dev, int32_t max_iter, double tolerance, double* elbo_traces, double* mse_traces,
+                   int32_t* n_done, int32_t n_streams) {
+    return fit_batch<double>(n_fits, cfgs, Y_dev, Xm_dev, Xc_dev, max_iter, tolerance, elbo_traces, mse_traces, n_done, n_streams);
+}
+int tame_fit_batch_f32(int32_t n_fits, const tame_config* cfgs, const float* const* Y_dev, double* const* Xm_dev,
+                       double* const* Xc_dev, int32_t max_iter, double tolerance, double* elbo_traces, double* mse_traces,
+                       int32_t* n_done, int32_t n_streams) {
+    return fit_batch<float>(n_fits, cfgs, Y_dev, Xm_dev, Xc_dev, max_iter, tolerance, elbo_traces, mse_traces, n_done, n_streams);
+}
+
 int tame_generate_Y(int32_t n, int32_t T, int32_t r, const double R[4], const double* X_dev, uint64_t seed,
                     int32_t row_begin, int32_t row_end, double* Y_dev, void* stream) {
-    if (!R || !X_dev || !Y_dev || row_begin < 0 || row_end > n || row_end < row_begin) return fail(TAME_EINVAL, "bad argument");
-    if (R[0] <= 0) return fail(TAME_EINVAL, "R must be positive definite");
-    const double l00 = std::sqrt(R[0]), l10 = R[2] / l00, l11sq = R[3] - l10 * l10;
-    if (l11sq <= 0) return fail(TAME_EINVAL, "R must be positive definite");
-    const size_t total = (size_t)(row_end - row_begin) * n * T;
-    if (total == 0) return TAME_OK;
-    const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 64);
-    k_generate<<<blocks, 256, 0, (cudaStream_t)stream>>>(n, T, r, l00, l10, std::sqrt(l11sq), X_dev, seed, row_begin, row_end, Y_dev);
-    tame_count_launch(1);
-    CK(cudaGetLastError());
-    return TAME_OK;
+    return generate_Y<double>(n, T, r, R, X_dev, seed, row_begin, row_end, Y_dev, stream);
+}
+int tame_generate_Y_f32(int32_t n, int32_t T, int32_t r, const double R[4], const double* X_dev, uint64_t seed,
+                        int32_t row_begin, int32_t row_end, float* Y_dev, void* stream) {
+    return generate_Y<float>(n, T, r, R, X_dev, seed, row_begin, row_end, Y_dev, stream);
 }
 
 int tame_comm_unique_id(void* id128) {

@@ -6,9 +6,11 @@
 //   ELBO                src/inference/structured_mf.py:115-209, src/inference/naive_mf.py:89-191
 //   reconstruction MSE  src/models/temporal_ame.py:255-291, src/models/static_ame.py:189-238
 //
-// Data layout in HBM (all FP64, row-major):
-//   Y    (nloc, n, T, 2)   the reference layout; for a fixed row the (j,t) pairs are contiguous 16-byte dyads,
-//                          so a warp with lane <-> t streams 512 contiguous bytes per partner j.
+// Data layout in HBM (row-major; FP64 except Y, which may be FP32):
+//   Y    (nloc, n, T, 2)   the reference layout, stored as double or float (template parameter YT of every kernel that reads
+//                          it; each dyad is widened to FP64 right after the load, all arithmetic is FP64).  For a fixed row
+//                          the (j,t) pairs are contiguous 16-byte (8-byte) dyads, so a warp with lane <-> t streams 512
+//                          (256) contiguous bytes per partner j.
 //   Xm   (n, T, D)         D = 2 + 2R, x = [a, b, U(R), V(R)]
 //   Xc   (n, T, D, D)
 //   H    (nloc, T, 2R)     partner contraction  [ sum_j w0*V_j (R) , sum_j w1*U_j (R) ]  ("z order")
@@ -37,7 +39,7 @@
 struct TameParams {
     int n, T, nloc, world, rank, panel, mode;
     double lr, p0, p1, q;     // R_inv = [[p0,q],[q,p1]]
-    const double* Y;          // local rows
+    const void* Y;            // local rows, double or float (TameY<YT>::ptr)
     double* Xm;
     double* Xc;
     double* Craw;             // (nloc, T, D, D) raw covariance of the sweep (chain) -> k_covblend applies the rule + damping into Xc
@@ -69,6 +71,11 @@ struct TameParams {
 __device__ __forceinline__ double2 tame_ld_stream2(const double* p) {
     double2 v;
     asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ float2 tame_ld_stream2(const float* p) {
+    float2 v;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
     return v;
 }
 __device__ __forceinline__ double tame_ld_cg(const double* p) { return __ldcg(p); }
@@ -165,9 +172,46 @@ __device__ __forceinline__ void tame_cp_async16(void* smem_dst, const void* gsrc
     const int sz = valid ? 16 : 0;
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(d), "l"(gsrc), "r"(sz) : "memory");
 }
+// 8-byte variant (float dyads of Y): cp.async.cg only takes a cp-size of 16, so this one goes through L1 (.ca)
+__device__ __forceinline__ void tame_cp_async8(void* smem_dst, const void* gsrc, bool valid) {
+    const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
+    const int sz = valid ? 8 : 0;
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(d), "l"(gsrc), "r"(sz) : "memory");
+}
 __device__ __forceinline__ void tame_cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void tame_cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// Element type of Y: one dyad (y_ij, y_ji) is a V2 in HBM and in the shared-memory staging buffers; `wide` turns it into
+// the FP64 pair all arithmetic runs on (exact for float).  `bits` is the raw bit pattern (mirror check / hash).
+template <class YT>
+struct TameY;
+template <>
+struct TameY<double> {
+    using V2 = double2;
+    static __host__ __device__ __forceinline__ const double* ptr(const TameParams& P) { return static_cast<const double*>(P.Y); }
+    static __device__ __forceinline__ void cp_async(void* dst, const double* src, bool valid) { tame_cp_async16(dst, src, valid); }
+    static __device__ __forceinline__ double2 ld_stream(const double* p) { return tame_ld_stream2(p); }
+    static __device__ __forceinline__ double2 wide(const double2& v) { return v; }
+    static __device__ __forceinline__ double2 lds(const double2* p) { return *p; }
+    static __device__ __forceinline__ unsigned long long bits(double v) { return (unsigned long long)__double_as_longlong(v); }
+};
+template <>
+struct TameY<float> {
+    using V2 = float2;
+    static __host__ __device__ __forceinline__ const float* ptr(const TameParams& P) { return static_cast<const float*>(P.Y); }
+    static __device__ __forceinline__ void cp_async(void* dst, const float* src, bool valid) { tame_cp_async8(dst, src, valid); }
+    static __device__ __forceinline__ float2 ld_stream(const float* p) { return tame_ld_stream2(p); }
+    static __device__ __forceinline__ double2 wide(const float2& v) { return make_double2((double)v.x, (double)v.y); }
+    // a ring slot read where it is used (an ordered shared load): left to itself the compiler hoists the cheaper float
+    // loads of later partners and the widened values then exceed the streaming loop's register budget at r = 8
+    static __device__ __forceinline__ double2 lds(const float2* p) {
+        float2 v;
+        asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"((unsigned)__cvta_generic_to_shared(p)));
+        return wide(v);
+    }
+    static __device__ __forceinline__ unsigned long long bits(float v) { return (unsigned long long)__float_as_uint(v); }
+};
 
 // shared-memory stride (doubles) of one staged X_mean record: D, or D+2 when D/2 is even, so that the 8 lanes of
 // a quarter-warp reading 16-byte pieces of consecutive records hit distinct bank groups
@@ -178,14 +222,14 @@ struct TameRec {
 
 // Streaming tile shared by k_contract and k_llmse.
 //   CTA = 8 warps; lane <-> time step t (32 consecutive t: 512 contiguous bytes of Y per partner), warp <-> RW rows.
-//   Y goes global -> shared through a per-thread ring of PD partners (cp.async, RW*PD 16-byte copies in flight
-//   per thread, 128 KB per CTA at RW=4): every thread later reads back exactly the dyads it copied, so the ring
+//   Y goes global -> shared through a per-thread ring of PD partners (cp.async, RW*PD 16-byte (float Y: 8-byte) copies in
+//   flight per thread, 128 KB (64 KB) per CTA at RW=4): every thread later reads back exactly the dyads it copied, so the ring
 //   needs no block-level synchronisation.  The partners' X_mean records (a,b,U,V at the CTA's 32 time steps) are
 //   staged in their natural layout, JC partners per chunk, double buffered, one __syncthreads per chunk.
-template <int R, int RW>
+template <int R, int RW, class YT = double>
 struct TameStream {
     static constexpr int D = 2 + 2 * R, JC = 8, PD = 8, RS = TameRec<D>::RS, PIECES = D / 2;
-    static constexpr size_t Y_BYTES = (size_t)PD * RW * 256 * sizeof(double2);
+    static constexpr size_t Y_BYTES = (size_t)PD * RW * 256 * sizeof(typename TameY<YT>::V2);
     static constexpr size_t M_BYTES = (size_t)2 * JC * 32 * RS * sizeof(double);
     static constexpr size_t SMEM = Y_BYTES + M_BYTES;
 };
@@ -196,15 +240,16 @@ struct TameStream {
 // w0 = p0*y0 + q*y1, w1 = q*y0 + p1*y1  -- the [U,V] rows of sum_j J'R^-1 y_ij (structured_mf.py:324).
 // Software pipeline described at TameStream.  Must be called by all 256 threads of the CTA.
 // ------------------------------------------------------------------------------------------------------
-template <int R, int RW>
-__device__ __forceinline__ void tame_stream_cols(const TameParams& P, unsigned char* smem_raw, const double* const (&yrow)[RW],
+template <int R, int RW, class YT>
+__device__ __forceinline__ void tame_stream_cols(const TameParams& P, unsigned char* smem_raw, const YT* const (&yrow)[RW],
                                                  const bool (&rv)[RW], int kw, int t0, int jb, int je, bool tri,
                                                  double (&accA)[RW][R], double (&accB)[RW][R], int* cursor = nullptr,
                                                  bool lane_on = true) {
-    using TS = TameStream<R, RW>;
+    using TS = TameStream<R, RW, YT>;
+    using Y2 = typename TameY<YT>::V2;
     constexpr int D = TS::D, JC = TS::JC, PD = TS::PD, RS = TS::RS;
     static_assert(JC == PD, "ring slot == position in chunk");
-    double2 (*Yr)[RW][256] = reinterpret_cast<double2 (*)[RW][256]>(smem_raw);                       // [PD][RW][256]
+    Y2 (*Yr)[RW][256] = reinterpret_cast<Y2 (*)[RW][256]>(smem_raw);                                 // [PD][RW][256]
     double (*Mb)[JC][32][RS] = reinterpret_cast<double (*)[JC][32][RS]>(smem_raw + TS::Y_BYTES);     // [2][JC][32][RS]
     const int tid = threadIdx.x, lane = tid & 31;
     const size_t jstride = (size_t)P.T * 2;
@@ -216,7 +261,7 @@ __device__ __forceinline__ void tame_stream_cols(const TameParams& P, unsigned c
         for (int rr = 0; rr < RW; ++rr) {
             const int k = kw + rr;
             const bool ok = lane_on && rv[rr] && (j < je) && (tri ? (j > k) : (j != k));
-            tame_cp_async16(&Yr[slot][rr][tid], yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
+            TameY<YT>::cp_async(&Yr[slot][rr][tid], yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
         }
     };
     // fast path of the record staging: with the natural record pitch (RS == D) and a full 32-step slice, partner j's records
@@ -267,7 +312,7 @@ __device__ __forceinline__ void tame_stream_cols(const TameParams& P, unsigned c
             double w0[RW], w1[RW];
 #pragma unroll
             for (int rr = 0; rr < RW; ++rr) {
-                const double2 y = Yr[jj][rr][tid];
+                const double2 y = TameY<YT>::lds(&Yr[jj][rr][tid]);
                 w0[rr] = P.p0 * y.x + P.q * y.y;
                 w1[rr] = P.q * y.x + P.p1 * y.y;
             }
@@ -294,9 +339,9 @@ __device__ __forceinline__ void tame_stream_cols(const TameParams& P, unsigned c
 // multi-GPU sweep's static upper part and right-looking pushes).  One pass over Y[k0:k1, j0:j1].
 // grid (ceil(T/32), ceil((k1-k0)/(8*RW))), block 256, TameStream::SMEM dynamic smem.
 // ------------------------------------------------------------------------------------------------------
-template <int R, int RW>
+template <int R, int RW, class YT>
 __global__ void __launch_bounds__(256, 1) k_contract(TameParams P, int k0, int k1, int j0, int j1, int tri, int accumulate) {
-    constexpr int NV = 2 * R, JC = TameStream<R, RW>::JC, RT = 8 * RW;
+    constexpr int NV = 2 * R, JC = TameStream<R, RW, YT>::JC, RT = 8 * RW;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int t0 = blockIdx.x * 32, t = t0 + lane;
@@ -310,17 +355,17 @@ __global__ void __launch_bounds__(256, 1) k_contract(TameParams P, int k0, int k
     for (int rr = 0; rr < RW; ++rr)
 #pragma unroll
         for (int a = 0; a < R; ++a) accA[rr][a] = accB[rr][a] = 0.0;
-    const double* yrow[RW];
+    const YT* yrow[RW];
     bool rv[RW];
 #pragma unroll
     for (int rr = 0; rr < RW; ++rr) {
         const int k = kw + rr;
         rv[rr] = (k < k1) && tv;
         const int l = tame_lrow(min(k, P.n - 1), P.panel, P.world);
-        yrow[rr] = P.Y + ((size_t)l * P.n * P.T + (tv ? t : 0)) * 2;
+        yrow[rr] = TameY<YT>::ptr(P) + ((size_t)l * P.n * P.T + (tv ? t : 0)) * 2;
     }
     const int jstart = tri ? max(j0, ((kbase + 1) / JC) * JC) : j0;
-    tame_stream_cols<R, RW>(P, smem_raw, yrow, rv, kw, t0, jstart, j1, tri != 0, accA, accB);
+    tame_stream_cols<R, RW, YT>(P, smem_raw, yrow, rv, kw, t0, jstart, j1, tri != 0, accA, accB);
 #pragma unroll
     for (int rr = 0; rr < RW; ++rr) {
         const int k = kw + rr;
@@ -464,7 +509,7 @@ __device__ __forceinline__ double tame_logdet_spd(double (&col)[D], double* rb2 
 #define TAME_WATCHDOG_NS 4000000000ull
 enum { TAME_ROLE_ALL = 0, TAME_ROLE_TOTALS = 1, TAME_ROLE_INPUT = 2 };
 
-template <int R, int NH>
+template <int R, int NH, class YT = double>
 struct __align__(16) TameChainSmem {
     static constexpr int D = 2 + 2 * R, NV = 2 * R, TOT = TameTot<R>::TOT, DP = D + 1;
     static constexpr int NSLOT = (NH == 1) ? 8 : 16;   // staging ring of the input side (power of two)
@@ -472,7 +517,7 @@ struct __align__(16) TameChainSmem {
     static constexpr int RING = (NH == 1) ? TAME_RING : 2 * TAME_RING;   // rows of the z ring (>= WMAX + look-ahead, power of two)
     static constexpr int NTS = (NH == 1) ? 1 : 8;      // staging ring of the totals warp (NH = 2)
     struct Stage {                                  // one node's global inputs (cp.async destinations, 16-byte aligned)
-        double2 ywin[WMAX];                    // Y[i, wlo + s, t, :] of the inline window
+        typename TameY<YT>::V2 ywin[WMAX];          // Y[i, wlo + s, t, :] of the inline window
         double2 hand[D];                            // hand-over slot {new mean, tag} of (i, t-1); foreign nodes (NH = 1): of (i, t)
         double mold[D], mnext[D];                   // old means of (i,t) and (i,t+1)
         double H[TAME_MAX_PARTS][NV];               // static partner part (per column part)
@@ -505,7 +550,8 @@ struct __align__(16) TameChainSmem {
     int pad_;
 };
 static_assert(sizeof(TameChainSmem<1, 1>) % 16 == 0 && sizeof(TameChainSmem<2, 1>) % 16 == 0 && sizeof(TameChainSmem<3, 1>) % 16 == 0 &&
-              sizeof(TameChainSmem<4, 2>) % 16 == 0 && sizeof(TameChainSmem<8, 2>) % 16 == 0, "per-time-step chain block must stay 16-byte aligned");
+              sizeof(TameChainSmem<4, 2>) % 16 == 0 && sizeof(TameChainSmem<8, 2>) % 16 == 0 &&
+              sizeof(TameChainSmem<1, 1, float>) % 16 == 0 && sizeof(TameChainSmem<3, 2, float>) % 16 == 0, "per-time-step chain block must stay 16-byte aligned");
 static_assert(TAME_LA + 2 <= 8 && 2 * (TAME_LA2 + 1) + 4 <= 16 && TAME_NL + 2 <= TAME_NINP, "mailbox depth");
 
 // panel-cyclic ownership of consecutive nodes without integer divisions: rem = k % panel, pw = (k / panel) % world,
@@ -593,10 +639,10 @@ __device__ __forceinline__ void tame_rank2_apply(double (&cw)[2 + 2 * R], const 
 // helper warp(s) of time step t.  ROLE_ALL: the one helper of NH = 1.  ROLE_TOTALS / ROLE_INPUT (hi = 0,1): the team of NH = 2;
 // an input warp takes the nodes i0 + hi, i0 + hi + 2, ...
 // ------------------------------------------------------------------------------------------------------
-template <int R, bool FUSED, int NH, int ROLE>
-__device__ __forceinline__ void tame_chain_helper(const TameParams& P, TameChainSmem<R, NH>& sm, const TameChainSmem<R, NH>* pv, int lane,
-                                                  int t, int hi, int i0, int i1) {
-    using S = TameChainSmem<R, NH>;
+template <int R, bool FUSED, int NH, int ROLE, class YT>
+__device__ __forceinline__ void tame_chain_helper(const TameParams& P, TameChainSmem<R, NH, YT>& sm, const TameChainSmem<R, NH, YT>* pv,
+                                                  int lane, int t, int hi, int i0, int i1) {
+    using S = TameChainSmem<R, NH, YT>;
     constexpr bool DO_TOT = (ROLE != TAME_ROLE_INPUT), DO_INP = (ROLE != TAME_ROLE_TOTALS);
     constexpr int STEP = (ROLE == TAME_ROLE_INPUT) ? NH : 1;
     constexpr int D = S::D, NV = S::NV, TOT = S::TOT, DP = S::DP;
@@ -707,11 +753,11 @@ __device__ __forceinline__ void tame_chain_helper(const TameParams& P, TameChain
         if (has_prev && act) tame_cp_async16(&s.hand[c], hand_prev + (size_t)k * T * D, true);
         if (has_next && lane >= 16 && lane < 16 + D / 2) tame_cp_async16(&s.mnext[2 * (lane - 16)], xm + D + 2 * (lane - 16), true);
         const int wlo = window_lo(k);
-        const double* yb = P.Y + (((size_t)l * P.n + wlo) * T + t) * 2;
+        const YT* yb = TameY<YT>::ptr(P) + (((size_t)l * P.n + wlo) * T + t) * 2;
 #pragma unroll
         for (int u = 0; u < NWS; ++u) {
             const int sl = lane + 32 * u;
-            if (wlo + sl < k) tame_cp_async16(&s.ywin[sl], yb + (size_t)sl * T * 2, true);
+            if (wlo + sl < k) TameY<YT>::cp_async(&s.ywin[sl], yb + (size_t)sl * T * 2, true);
         }
         if (FUSED && ((k % TAME_SB) < STEP)) {                   // this warp's first node of the sub-block
             const long long c0 = clock64();
@@ -809,7 +855,7 @@ __device__ __forceinline__ void tame_chain_helper(const TameParams& P, TameChain
                 for (int u = 0; u < NWS; ++u) {
                     const int sl = lane + 32 * u;
                     if (wlo + sl < k) {
-                        const double2 y = s.ywin[sl];
+                        const double2 y = TameY<YT>::wide(s.ywin[sl]);
                         wbuf[sl] = make_double2(P.p0 * y.x + P.q * y.y, P.q * y.x + P.p1 * y.y);
                     }
                 }
@@ -1032,9 +1078,9 @@ __device__ __forceinline__ void tame_chain_helper(const TameParams& P, TameChain
 // ------------------------------------------------------------------------------------------------------
 // chain warp of time step t
 // ------------------------------------------------------------------------------------------------------
-template <int R, bool FUSED, int NH>
-__device__ __forceinline__ void tame_chain_warp(const TameParams& P, TameChainSmem<R, NH>& sm, int lane, int t, int i0, int i1) {
-    using S = TameChainSmem<R, NH>;
+template <int R, bool FUSED, int NH, class YT>
+__device__ __forceinline__ void tame_chain_warp(const TameParams& P, TameChainSmem<R, NH, YT>& sm, int lane, int t, int i0, int i1) {
+    using S = TameChainSmem<R, NH, YT>;
     constexpr int D = S::D, NV = S::NV, DP = S::DP;
     constexpr int NL = TAME_NL, IMASK = TAME_NINP - 1, RMASK = S::RING - 1;
     const int T = P.T, c = lane, cc = min(c, D - 1);
@@ -1229,9 +1275,9 @@ template <int NH>
 struct TameTeam {
     static constexpr int TPC = (NH == 1) ? 4 : 2;        // time steps per chain CTA
 };
-template <int R, bool FUSED, int NH>
+template <int R, bool FUSED, int NH, class YT>
 __device__ __forceinline__ void tame_chain_body(const TameParams& P, unsigned char* smem_raw, int cta, int i0, int i1) {
-    using S = TameChainSmem<R, NH>;
+    using S = TameChainSmem<R, NH, YT>;
     constexpr int TPC = TameTeam<NH>::TPC;
     S* team = reinterpret_cast<S*>(smem_raw);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1247,8 +1293,8 @@ __device__ __forceinline__ void tame_chain_body(const TameParams& P, unsigned ch
         if (tg >= TPC) return;
         const int t = cta * TPC + tg;
         if (t >= P.T) return;
-        if (is_helper) tame_chain_helper<R, FUSED, NH, TAME_ROLE_ALL>(P, team[tg], (tg > 0) ? &team[tg - 1] : nullptr, lane, t, 0, i0, i1);
-        else tame_chain_warp<R, FUSED, NH>(P, team[tg], lane, t, i0, i1);
+        if (is_helper) tame_chain_helper<R, FUSED, NH, TAME_ROLE_ALL, YT>(P, team[tg], (tg > 0) ? &team[tg - 1] : nullptr, lane, t, 0, i0, i1);
+        else tame_chain_warp<R, FUSED, NH, YT>(P, team[tg], lane, t, i0, i1);
     } else {
         const int tg = warp >> 2;
         if (tg >= TPC) return;
@@ -1256,9 +1302,9 @@ __device__ __forceinline__ void tame_chain_body(const TameParams& P, unsigned ch
         const int t = cta * TPC + tg;
         if (t >= P.T) return;
         const S* pv = (tg > 0) ? &team[tg - 1] : nullptr;
-        if (role == 0) tame_chain_warp<R, FUSED, NH>(P, team[tg], lane, t, i0, i1);
-        else if (role == 1) tame_chain_helper<R, FUSED, NH, TAME_ROLE_TOTALS>(P, team[tg], pv, lane, t, 0, i0, i1);
-        else tame_chain_helper<R, FUSED, NH, TAME_ROLE_INPUT>(P, team[tg], pv, lane, t, role - 2, i0, i1);
+        if (role == 0) tame_chain_warp<R, FUSED, NH, YT>(P, team[tg], lane, t, i0, i1);
+        else if (role == 1) tame_chain_helper<R, FUSED, NH, TAME_ROLE_TOTALS, YT>(P, team[tg], pv, lane, t, 0, i0, i1);
+        else tame_chain_helper<R, FUSED, NH, TAME_ROLE_INPUT, YT>(P, team[tg], pv, lane, t, role - 2, i0, i1);
     }
 }
 
@@ -1320,10 +1366,10 @@ __global__ void __launch_bounds__(256) k_covblend(TameParams P) {
 }
 
 // stand-alone chain launch over one 64-node block (multi-GPU path); cooperative, grid = ceil(T/8)
-template <int R>
+template <int R, class YT>
 __global__ void __launch_bounds__(2 * TAME_CHAIN_WPC * 32, 1) k_chain(TameParams P, int i0, int i1) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    tame_chain_body<R, false, 1>(P, smem_raw, blockIdx.x, i0, i1);
+    tame_chain_body<R, false, 1, YT>(P, smem_raw, blockIdx.x, i0, i1);
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -1339,14 +1385,14 @@ __global__ void __launch_bounds__(2 * TAME_CHAIN_WPC * 32, 1) k_chain(TameParams
 // Every Y entry is read exactly once per sweep; the schedule is the reference's.
 // grid = n_chain_ctas + workers (all co-resident), block 256, dynamic smem = max of the two roles.
 // ------------------------------------------------------------------------------------------------------
-template <int R, int RW, int NH>
+template <int R, int RW, int NH, class YT>
 __device__ __forceinline__ void tame_sweep_body(const TameParams& P, unsigned char* smem_raw) {
     static_assert(8 * RW == TAME_SB, "a streaming unit is one sub-block of rows");
     if ((int)blockIdx.x < P.n_chain_ctas) {
-        tame_chain_body<R, true, NH>(P, smem_raw, blockIdx.x, 0, P.n);
+        tame_chain_body<R, true, NH, YT>(P, smem_raw, blockIdx.x, 0, P.n);
         return;
     }
-    constexpr int NV = 2 * R, JC = TameStream<R, RW>::JC;
+    constexpr int NV = 2 * R, JC = TameStream<R, RW, YT>::JC;
     __shared__ int s_val;
     __shared__ int s_dg[TAME_NG], s_plan[3];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1368,13 +1414,13 @@ __device__ __forceinline__ void tame_sweep_body(const TameParams& P, unsigned ch
         for (int rr = 0; rr < RW; ++rr)
 #pragma unroll
             for (int a = 0; a < R; ++a) accA[rr][a] = accB[rr][a] = 0.0;
-        const double* yrow[RW];
+        const YT* yrow[RW];
         bool rv[RW];
 #pragma unroll
         for (int rr = 0; rr < RW; ++rr) {
             const int k = kw + rr;
             rv[rr] = (k < P.n) && tv;
-            yrow[rr] = P.Y + ((size_t)tame_lrow(min(k, P.n - 1), P.panel, P.world) * P.n * P.T + (tv ? t : 0)) * 2;
+            yrow[rr] = TameY<YT>::ptr(P) + ((size_t)tame_lrow(min(k, P.n - 1), P.panel, P.world) * P.n * P.T + (tv ? t : 0)) * 2;
         }
         // optional trace of the unit (sub-block, slice 0, part 0): claim, upper part done, group 0 urgent, group 0 stamped
         unsigned long long* utr = (P.trace != nullptr && slice == 0 && part == P.nparts - 1 && tid == 0) ? P.trace + 2 * nsb + 4 * lsb : nullptr;
@@ -1395,8 +1441,8 @@ __device__ __forceinline__ void tame_sweep_body(const TameParams& P, unsigned ch
                 __syncthreads();
                 if (cur > jb && cur < je) start = jb + ((cur - jb) / JC) * JC;
             }
-            tame_stream_cols<R, RW>(P, smem_raw, yrow, rv, kw, t0, start, je, true, accA, accB, P.cursor + part);
-            if (start > jb) tame_stream_cols<R, RW>(P, smem_raw, yrow, rv, kw, t0, jb, start, true, accA, accB, P.cursor + part);
+            tame_stream_cols<R, RW, YT>(P, smem_raw, yrow, rv, kw, t0, start, je, true, accA, accB, P.cursor + part);
+            if (start > jb) tame_stream_cols<R, RW, YT>(P, smem_raw, yrow, rv, kw, t0, jb, start, true, accA, accB, P.cursor + part);
         }
         // (b) lower columns, released by the chain (carried by part 0).  The unit's 32 time steps are followed as TAME_NG
         // groups of 8: the chain warps of a slice are skewed by ~2 us per time step, so the first group of a slice reaches
@@ -1493,17 +1539,17 @@ __device__ __forceinline__ void tame_sweep_body(const TameParams& P, unsigned ch
             if (c0 == -2) break;                             // abort: leave without stamping
             if (c0 < 0) { __nanosleep(128); continue; }
             const bool lane_on = (mask >> (lane >> 3)) & 1;      // lanes of the other groups copy nothing and add zeros
-            tame_stream_cols<R, RW>(P, smem_raw, yrow, rv, kw, t0, c0, c1, false, accA, accB, nullptr, lane_on);
+            tame_stream_cols<R, RW, YT>(P, smem_raw, yrow, rv, kw, t0, c0, c1, false, accA, accB, nullptr, lane_on);
             if (tid < TAME_NG && ((mask >> tid) & 1)) s_dg[tid] = c1;
             __syncthreads();
         }
     }
 }
 
-template <int R, int RW, int NH>
+template <int R, int RW, int NH, class YT>
 __global__ void __launch_bounds__(256, 1) k_sweep(TameParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    tame_sweep_body<R, RW, NH>(P, smem_raw);
+    tame_sweep_body<R, RW, NH, YT>(P, smem_raw);
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -1520,14 +1566,15 @@ __global__ void __launch_bounds__(256, 1) k_sweep(TameParams P) {
 // SYM: Y was verified mirror-consistent at bind time (Y[j,i,t,:] == swap(Y[i,j,t,:]) bit for bit, which the reference's
 // generate_data guarantees, temporal_ame.py:209-216): the residuals of (j,i) are those of (i,j) swapped, so the pass only
 // streams the partners j > i and doubles the squared error.  Otherwise the full pass runs.
-template <int R, int RW, int NW, bool SYM>
+template <int R, int RW, int NW, bool SYM, class YT>
 __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* partial) {
-    using TS = TameStream<R, RW>;
+    using TS = TameStream<R, RW, YT>;
+    using Y2 = typename TameY<YT>::V2;
     constexpr int D = TS::D, JC = TS::JC, PD = TS::PD, RS = TS::RS, RT = NW * RW, NT = NW * 32;
     static_assert(NW * RW == 32, "32-row tile");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    double2 (*Yr)[RW][NT] = reinterpret_cast<double2 (*)[RW][NT]>(smem_raw);
-    double (*Mb)[JC][32][RS] = reinterpret_cast<double (*)[JC][32][RS]>(smem_raw + (size_t)PD * RW * NT * sizeof(double2));
+    Y2 (*Yr)[RW][NT] = reinterpret_cast<Y2 (*)[RW][NT]>(smem_raw);
+    double (*Mb)[JC][32][RS] = reinterpret_cast<double (*)[JC][32][RS]>(smem_raw + (size_t)PD * RW * NT * sizeof(Y2));
     __shared__ double red[2][NW];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int t0 = blockIdx.x * 32, t = t0 + lane;
@@ -1535,7 +1582,7 @@ __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* part
     const int lw = blockIdx.y * RT + warp * RW;
 
     double oa[RW], ob[RW], oU[RW][R], oV[RW][R];
-    const double* yrow[RW];
+    const YT* yrow[RW];
     int gi[RW];
     bool rv[RW];
 #pragma unroll
@@ -1549,7 +1596,7 @@ __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* part
         ob[rr] = m[1];
 #pragma unroll
         for (int a = 0; a < R; ++a) { oU[rr][a] = m[2 + a]; oV[rr][a] = m[2 + R + a]; }
-        yrow[rr] = P.Y + ((size_t)l * P.n * P.T + (tv ? t : 0)) * 2;
+        yrow[rr] = TameY<YT>::ptr(P) + ((size_t)l * P.n * P.T + (tv ? t : 0)) * 2;
     }
     const size_t jstride = (size_t)P.T * 2;
     // per-row moment accumulators: upper partners (j > i) feed S00 = sum e0^2, S01 = sum e0 e1, S11 = sum e1^2 (the
@@ -1570,7 +1617,7 @@ __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* part
 #pragma unroll
         for (int rr = 0; rr < RW; ++rr) {
             const bool ok = rv[rr] && (j < jend) && (SYM ? (j > gi[rr]) : (j != gi[rr]));
-            tame_cp_async16(&Yr[slot][rr][tid], yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
+            TameY<YT>::cp_async(&Yr[slot][rr][tid], yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
         }
     };
     // fast path of the record staging (see tame_stream_cols)
@@ -1632,7 +1679,7 @@ __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* part
             }
 #pragma unroll
             for (int rr = 0; rr < RW; ++rr) {
-                const double2 y = Yr[jj][rr][tid];
+                const double2 y = TameY<YT>::wide(Yr[jj][rr][tid]);
                 const double e0 = y.x - d0[rr], e1 = y.y - d1[rr];
                 if (kind == 1) {
                     S00[rr] = fma(e0, e0, S00[rr]);
@@ -1687,7 +1734,8 @@ __global__ void __launch_bounds__(NW * 32, 1) k_llmse(TameParams P, double* part
 //   For a fixed time step the 8x8 blocks  d0[i][j] = U_i.V_j  and  d1[i][j] = V_i.U_j  of an (8 rows x 8 partners) tile
 //   are R/4 DMMA each: A = the tile's own rows (kept in registers for the whole pass), B = the partners' records staged
 //   in shared memory.  The accumulator fragment gives every lane two dyads (row g, partners 2q, 2q+1), whose Y entries
-//   it reads from the cp.async ring (padded pitches 517/257 so that a quarter-warp's 16-byte reads hit distinct banks).
+//   it reads from the cp.async ring (padded pitches 517/257 so that a quarter-warp's 16-byte reads hit distinct banks; the
+//   float-Y ring keeps the same pitches in 8-byte units).
 //   CTA = 8 warps = 16 rows x 32 time steps; warp w owns time steps t0+4w..+3 and both 8-row tiles.  ~0.36 issued
 //   instructions per dyad instead of ~1.25.  R must be a multiple of 4.
 // grid (ceil(T/32), ceil(nloc/16)), block 256; partial (grid.y*grid.x, 2).
@@ -1696,23 +1744,24 @@ __device__ __forceinline__ void tame_dmma(double& c0, double& c1, double a, doub
     asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-template <int R>
+template <int R, class YT = double>
 struct TameMma {
     static constexpr int D = 2 + 2 * R, JC = 8, RS = TameRec<D>::RS, PIECES = D / 2, KS = R / 4;
-    static constexpr int PR = 257, PJ = 517;                       // ring pitches in 16-byte units (see header)
+    static constexpr int PR = 257, PJ = 517;                       // ring pitches in dyads (see header)
     static constexpr int MJ = 32 * RS + 4;                         // partner pitch of the staged records (doubles)
-    static constexpr size_t Y_BYTES = (size_t)2 * JC * PJ * sizeof(double2);
+    static constexpr size_t Y_BYTES = (size_t)2 * JC * PJ * sizeof(typename TameY<YT>::V2);
     static constexpr size_t M_BYTES = (size_t)2 * JC * MJ * sizeof(double);
     static constexpr size_t SMEM = Y_BYTES + M_BYTES;
 };
 
-template <int R, bool SYM>
+template <int R, bool SYM, class YT>
 __global__ void __launch_bounds__(256, 1) k_llmse_mma(TameParams P, double* partial) {
-    using TM = TameMma<R>;
+    using TM = TameMma<R, YT>;
+    using Y2 = typename TameY<YT>::V2;
     constexpr int D = TM::D, JC = TM::JC, RS = TM::RS, KS = TM::KS, PR = TM::PR, PJ = TM::PJ, MJ = TM::MJ, RT = 16;
     static_assert(R % 4 == 0, "DMMA k-step is 4");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    double2* Yr = reinterpret_cast<double2*>(smem_raw);                          // [2][JC*PJ]
+    Y2* Yr = reinterpret_cast<Y2*>(smem_raw);                                    // [2][JC*PJ]
     double* Mb = reinterpret_cast<double*>(smem_raw + TM::Y_BYTES);              // [2][JC*MJ]
     __shared__ double red[2][8];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1722,7 +1771,7 @@ __global__ void __launch_bounds__(256, 1) k_llmse_mma(TameParams P, double* part
     const int gfirst = tame_grow(min(lrow0, P.nloc - 1), P.panel, P.world, P.rank);   // first node of the tile (16 | panel)
 
     // ---- copy role: this thread moves the dyads of rows lrow0 + 2*warp + {0,1} at time t0 + lane
-    const double* yrow[2];
+    const YT* yrow[2];
     bool rvc[2];
     int gic[2];
 #pragma unroll
@@ -1731,18 +1780,18 @@ __global__ void __launch_bounds__(256, 1) k_llmse_mma(TameParams P, double* part
         rvc[rr] = (l < P.nloc) && (t0 + lane < P.T);
         l = min(l, P.nloc - 1);
         gic[rr] = tame_grow(l, P.panel, P.world, P.rank);
-        yrow[rr] = P.Y + ((size_t)l * P.n * P.T + min(t0 + lane, P.T - 1)) * 2;
+        yrow[rr] = TameY<YT>::ptr(P) + ((size_t)l * P.n * P.T + min(t0 + lane, P.T - 1)) * 2;
     }
     const size_t jstride = (size_t)P.T * 2;
     auto issue_chunk = [&](int buf, int jc) {
-        double2* yb = Yr + (size_t)buf * JC * PJ;
+        Y2* yb = Yr + (size_t)buf * JC * PJ;
 #pragma unroll
         for (int jj = 0; jj < JC; ++jj) {
             const int j = jc + jj;
 #pragma unroll
             for (int rr = 0; rr < 2; ++rr) {
                 const bool ok = rvc[rr] && (j < P.n) && (SYM ? (j > gic[rr]) : (j != gic[rr]));
-                tame_cp_async16(yb + jj * PJ + rr * PR + tid, yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
+                TameY<YT>::cp_async(yb + jj * PJ + rr * PR + tid, yrow[rr] + (size_t)min(j, P.n - 1) * jstride, ok);
             }
         }
         double* mb = Mb + (size_t)buf * JC * MJ;
@@ -1789,7 +1838,7 @@ __global__ void __launch_bounds__(256, 1) k_llmse_mma(TameParams P, double* part
         const int jc = jbeg + c * JC, buf = c & 1;
         if (c + 1 < nchunks) tame_cp_async_wait<1>(); else tame_cp_async_wait<0>();
         __syncthreads();                                       // chunk c (Y dyads + partner records) is visible to the CTA
-        const double2* yb = Yr + (size_t)buf * JC * PJ;
+        const Y2* yb = Yr + (size_t)buf * JC * PJ;
         const double* mb = Mb + (size_t)buf * JC * MJ;
         // 0: all partners below the tile's rows, 1: all above (and inside the matrix), 2: mixed / tail
         const int kind = (jc + JC <= gfirst) ? 0 : ((jc > gfirst + RT - 1 && jc + JC <= P.n) ? 1 : 2);
@@ -1818,8 +1867,8 @@ __global__ void __launch_bounds__(256, 1) k_llmse_mma(TameParams P, double* part
                 }
                 // the two dyads of this lane: row (8*tile + g) -> copied by warp (4*tile + g/2), rr = g & 1
                 const int slot = (g & 1) * PR + (4 * tile + (g >> 1)) * 32 + tl;
-                const double2 y0 = yb[(2 * q) * PJ + slot];
-                const double2 y1 = yb[(2 * q + 1) * PJ + slot];
+                const double2 y0 = TameY<YT>::wide(yb[(2 * q) * PJ + slot]);
+                const double2 y1 = TameY<YT>::wide(yb[(2 * q + 1) * PJ + slot]);
                 const int gi = grow[tile];
                 const double e00 = y0.x - ((oa[tt][tile] + ab0.y) + d00), e01 = y0.y - ((ab0.x + ob[tt][tile]) + d10);
                 const double e10 = y1.x - ((oa[tt][tile] + ab1.y) + d01), e11 = y1.y - ((ab1.x + ob[tt][tile]) + d11);
@@ -2070,7 +2119,7 @@ __device__ __forceinline__ void tame_totals_small(const TameParams& P, double* r
 // time slice), lane <-> (t, partner subgroup): W = 8, 16 or 32 time steps per slice, whichever pads T least, and the 32 / W
 // lane groups take every (32/W)-th partner (a short T would otherwise leave most lanes idle).  Fixed summation order
 // (structured_mf.py:124-146, temporal_ame.py:255-291); per-block sums -> part[bid][0..1]
-template <int R>
+template <int R, class YT>
 __device__ __forceinline__ void tame_llmse_small(const TameParams& P, double* part, double* red /* 16 doubles smem */, int bid, int nb) {
     constexpr int D = 2 + 2 * R;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -2088,7 +2137,7 @@ __device__ __forceinline__ void tame_llmse_small(const TameParams& P, double* pa
             double ai = mi[0], bi = mi[1], Ui[R], Vi[R];
 #pragma unroll
             for (int a = 0; a < R; ++a) { Ui[a] = mi[2 + a]; Vi[a] = mi[2 + R + a]; }
-            const double* yrow = P.Y + ((size_t)i * P.n * P.T + t) * 2;
+            const YT* yrow = TameY<YT>::ptr(P) + ((size_t)i * P.n * P.T + t) * 2;
             double s = 0.0, q = 0.0;
             // partners four at a time: the loads of a group are issued before the first use (L2 latency, no ring here)
             for (int j0 = js; j0 < P.n; j0 += 4 * G) {
@@ -2097,7 +2146,7 @@ __device__ __forceinline__ void tame_llmse_small(const TameParams& P, double* pa
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     const int j = min(j0 + u * G, P.n - 1);
-                    y[u] = tame_ld_stream2(yrow + (size_t)j * P.T * 2);
+                    y[u] = TameY<YT>::wide(TameY<YT>::ld_stream(yrow + (size_t)j * P.T * 2));
                     const double* mj = P.Xm + ((size_t)j * P.T + t) * D;
 #pragma unroll
                     for (int k = 0; k < D; ++k) rec[u][k] = __ldcg(mj + k);
@@ -2136,7 +2185,7 @@ __device__ __forceinline__ void tame_llmse_small(const TameParams& P, double* pa
     __syncthreads();
 }
 
-template <int R, int RW, int NH>
+template <int R, int RW, int NH, class YT>
 __global__ void __launch_bounds__(256, 1) k_fit(TameParams P0, TameFitArgs F) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int D = 2 + 2 * R;
@@ -2155,14 +2204,14 @@ __global__ void __launch_bounds__(256, 1) k_fit(TameParams P0, TameFitArgs F) {
         }
         tame_grid_sync(F.bar, nblk, phase);
         // ---- the sweep: chain CTAs + streaming CTAs, exactly as in k_sweep
-        tame_sweep_body<R, RW, NH>(P, smem_raw);
+        tame_sweep_body<R, RW, NH, YT>(P, smem_raw);
         tame_grid_sync(F.bar, nblk, phase);
         // ---- factorisation rule + damped write of the covariance blocks
         tame_covblend_impl<R>(P, reinterpret_cast<double*>(smem_raw), bid, (int)nblk);
         tame_grid_sync(F.bar, nblk, phase);
         // ---- ELBO / MSE partial sums
         tame_cellterms_impl<R>(P, F.logdetS0, F.logdetQ, part4, *reinterpret_cast<TameCellSmem<R>*>(smem_raw), bid, (int)nblk);
-        tame_llmse_small<R>(P, F.part, reinterpret_cast<double*>(smem_raw), bid, (int)nblk);
+        tame_llmse_small<R, YT>(P, F.part, reinterpret_cast<double*>(smem_raw), bid, (int)nblk);
         tame_grid_sync(F.bar, nblk, phase);
         // ---- block 0: deterministic reduction, ELBO (k_finalize's formulas), the stop rule of base.py:183-203
         if (bid == 0) {
@@ -2201,24 +2250,30 @@ __global__ void __launch_bounds__(256, 1) k_fit(TameParams P0, TameFitArgs F) {
     }
 }
 
+// launchers of the kernels that read Y, for one element type of Y (each queries its own instantiation: the shared-memory
+// footprint depends on the type)
+struct TameYOps {
+    void (*contract)(const TameParams&, int k0, int k1, int j0, int j1, int tri, int accumulate, cudaStream_t);
+    cudaError_t (*chain)(const TameParams&, int i0, int i1, cudaStream_t);
+    cudaError_t (*sweep_fused)(const TameParams&, cudaStream_t);
+    cudaError_t (*fit_device)(const TameParams&, const TameFitArgs&, int* grid_out, cudaStream_t);
+    int (*fit_grid)(const TameParams&);
+    int (*sweep_capacity)(int nh);
+    void (*llmse)(const TameParams&, double* partial, int* nblocks, int symmetric, cudaStream_t);
+};
+
 // function table of one latent dimension
 struct TameOps {
     int r;
     size_t chain_smem;
     int tot;
     void (*totals)(const TameParams&, double* partial, int NS, cudaStream_t);
-    void (*contract)(const TameParams&, int k0, int k1, int j0, int j1, int tri, int accumulate, cudaStream_t);
-    cudaError_t (*chain)(const TameParams&, int i0, int i1, cudaStream_t);
     void (*covblend)(const TameParams&, cudaStream_t);
-    cudaError_t (*sweep_fused)(const TameParams&, cudaStream_t);
-    cudaError_t (*fit_device)(const TameParams&, const TameFitArgs&, int* grid_out, cudaStream_t);
-    int (*fit_grid)(const TameParams&);
-    int (*sweep_capacity)(int nh);
     int (*chain_max_T)();
-    void (*llmse)(const TameParams&, double* partial, int* nblocks, int symmetric, cudaStream_t);
     void (*cellterms)(const TameParams&, double logdetS0, double logdetQ, double* partial, int nblocks, cudaStream_t);
     int (*llmse_blocks)(const TameParams&);
     int (*cellterms_blocks)(const TameParams&);
+    TameYOps f64, f32;         // Y stored as double / as float
 };
 const TameOps* tame_get_ops(int r);
 void tame_count_launch(int n);

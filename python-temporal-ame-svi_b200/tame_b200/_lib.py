@@ -45,6 +45,7 @@ SIGNATURES = {
     "tame_set_stream": (C.c_int, [_P, _P]),
     "tame_local_rows": (C.c_int, [_P, C.POINTER(C.c_int32)]),
     "tame_bind_Y": (C.c_int, [_P, _P]),
+    "tame_bind_Y_f32": (C.c_int, [_P, _P]),
     "tame_bind_state": (C.c_int, [_P, _P, _P]),
     "tame_sweep": (C.c_int, [_P]),
     "tame_elbo_mse": (C.c_int, [_P, _DP]),
@@ -52,9 +53,13 @@ SIGNATURES = {
     "tame_fit": (C.c_int, [_P, C.c_int32, C.c_double, _DP, _DP, C.POINTER(C.c_int32)]),
     "tame_fit_device": (C.c_int, [_P, C.c_int32, C.c_double, _P, _P, _P]),
     "tame_fit_host": (C.c_int, [C.POINTER(TameConfig), _P, _P, _P, C.c_int32, C.c_double, _DP, _DP, C.POINTER(C.c_int32)]),
+    "tame_fit_host_f32": (C.c_int, [C.POINTER(TameConfig), _P, _P, _P, C.c_int32, C.c_double, _DP, _DP, C.POINTER(C.c_int32)]),
     "tame_fit_batch": (C.c_int, [C.c_int32, C.POINTER(TameConfig), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.c_int32,
                                 C.c_double, _DP, _DP, C.POINTER(C.c_int32), C.c_int32]),
+    "tame_fit_batch_f32": (C.c_int, [C.c_int32, C.POINTER(TameConfig), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.c_int32,
+                                    C.c_double, _DP, _DP, C.POINTER(C.c_int32), C.c_int32]),
     "tame_generate_Y": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _DP, _P, C.c_uint64, C.c_int32, C.c_int32, _P, _P]),
+    "tame_generate_Y_f32": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _DP, _P, C.c_uint64, C.c_int32, C.c_int32, _P, _P]),
     "tame_align_states": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P, _P, _DP, _P]),
     "tame_align_signs": (C.c_int, [C.c_int64, C.c_int32, _P, _P, _P, _DP, _P]),
     "tame_procrustes": (C.c_int, [C.c_int32, C.c_int32, _P, _P, C.c_int32, _P, _P, _P]),

@@ -7,6 +7,10 @@ the three calls of the fit loop run: `_update_step`, `_compute_elbo` and `_compu
 C-ABI calls into libtame_b200.so (hand-written sm_100a FP64 kernels).  There is no CPU fallback; without a CUDA
 device or without the built library these calls raise.
 
+Y is kept on the device in the dtype it arrives in when that is float32 (the reference's default), and widened to FP64
+by the kernels as they load it: half the HBM and host->device bytes, the same results bit for bit as a float64 copy
+of the same values.  Any other dtype is converted to float64 as before.
+
 Host/device protocol: the variational state lives in HBM while an engine exists; `vi.X_mean` / `vi.X_cov`
 are properties that read the device state back on access (and upload on assignment), so reference-style code
 that inspects or pickles the object keeps working.  Initialisation stays on the host and issues the reference's
@@ -24,6 +28,18 @@ import torch
 
 from . import _lib
 from .sharding import DEFAULT_PANEL, owned_rows
+
+
+def _device_Y(Y: torch.Tensor, dev: torch.device) -> torch.Tensor:
+    """Y on `dev` as float32 (kept as it is) or float64 (everything else), contiguous.  A contiguous float32 tensor
+    already on `dev` is returned as is: a second copy of the largest Y a GPU holds would not fit next to it."""
+    dt = torch.float32 if Y.dtype == torch.float32 else torch.float64
+    return Y.detach().to(dev, dt).contiguous()
+
+
+def _bind_Y(lib, handle, Y: torch.Tensor) -> int:
+    """tame_bind_Y or tame_bind_Y_f32, whichever matches Y's dtype (returns the C-ABI code)."""
+    return (lib.tame_bind_Y_f32 if Y.dtype == torch.float32 else lib.tame_bind_Y)(handle, Y.data_ptr())
 
 
 def _fit_config(vi, device_index: int, world: int = 1, rank: int = 0, panel: int = 0):
@@ -55,7 +71,8 @@ def _fit_config(vi, device_index: int, world: int = 1, rank: int = 0, panel: int
 
 
 class _Engine:
-    """Owns one libtame handle plus the device copies of Y / X_mean / X_cov (torch CUDA tensors, FP64)."""
+    """Owns one libtame handle plus the device copies of Y (float32 or FP64) / X_mean / X_cov (FP64) as torch CUDA
+    tensors."""
 
     def __init__(self, vi, device=None, world: int = 1, rank: int = 0, panel: int = 0):
         if not torch.cuda.is_available():
@@ -74,13 +91,13 @@ class _Engine:
         with torch.cuda.device(dev):
             _lib.check(self.lib.tame_create(C.byref(cfg), C.byref(self.handle)))
             Y = vi.Y if vi.Y is not None else model.Y
-            self.Y = Y.detach().to(dev, f64).contiguous()
+            self.Y = _device_Y(Y, dev)
             if tuple(self.Y.shape) != (n, n, T, 2):
                 raise ValueError(f"Y has shape {tuple(self.Y.shape)}, expected {(n, n, T, 2)}")
             self.X_mean = torch.empty(n, T, d, dtype=f64, device=dev)
             self.X_cov = torch.empty(n, T, d, d, dtype=f64, device=dev)
             torch.cuda.current_stream(dev).synchronize()
-            _lib.check(self.lib.tame_bind_Y(self.handle, self.Y.data_ptr()))
+            _lib.check(_bind_Y(self.lib, self.handle, self.Y))
             _lib.check(self.lib.tame_bind_state(self.handle, self.X_mean.data_ptr(), self.X_cov.data_ptr()))
         self._out6 = (C.c_double * 6)()
 
@@ -149,7 +166,7 @@ class _MultiEngine:
             h = C.c_void_p()
             with torch.cuda.device(dv):
                 _lib.check(self.lib.tame_create(C.byref(cfg), C.byref(h)))
-                self.Y.append(torch.cat([Yfull[a:b] for a, b in self.rows[rk]], 0).to(dv, f64).contiguous())
+                self.Y.append(_device_Y(torch.cat([Yfull[a:b] for a, b in self.rows[rk]], 0), dv))
                 self.Xm.append(torch.empty(n, T, d, dtype=f64, device=dv))
                 self.Xc.append(torch.empty(n, T, d, d, dtype=f64, device=dv))
                 torch.cuda.synchronize(dv)
@@ -161,7 +178,7 @@ class _MultiEngine:
         table = (C.c_void_p * self.world)(*[h.value for h in self.handles])
         for rk in range(self.world):
             _lib.check(self.lib.tame_peer_attach(self.handles[rk], table))
-        self._each(lambda rk: self.lib.tame_bind_Y(self.handles[rk], self.Y[rk].data_ptr()))
+        self._each(lambda rk: _bind_Y(self.lib, self.handles[rk], self.Y[rk]))
         for rk in range(self.world):
             _lib.check(self.lib.tame_bind_state(self.handles[rk], self.Xm[rk].data_ptr(), self.Xc[rk].data_ptr()))
         self._out6 = [(C.c_double * 6)() for _ in range(self.world)]
@@ -530,7 +547,8 @@ def fit_batch(vis, max_iter: int = 100, tolerance: float = 1e-4, device=None, n_
     verbose=False)` would give it -- history appended, state updated, per-fit early stop (base.py:183-203) -- but the
     fits run concurrently on one GPU.  `devices=[0, 1, ...]` deals the fits over several GPUs (independent fits, no
     collective: largest first to the least loaded device), one tame_fit_batch call per device from its own host thread.
-    Returns the list of histories."""
+    When every object's Y is float32 the fits keep float32 observations on the device (tame_fit_batch_f32); a batch
+    with any other dtype widens every Y to float64, which gives the same results.  Returns the list of histories."""
     if not torch.cuda.is_available():
         raise RuntimeError("tame_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
     vis = list(vis)
@@ -558,6 +576,8 @@ def fit_batch(vis, max_iter: int = 100, tolerance: float = 1e-4, device=None, n_
     cfgs = (_lib.TameConfig * nf)()
     Yp, Mp, Cp = (C.c_void_p * nf)(), (C.c_void_p * nf)(), (C.c_void_p * nf)()
     keep = []
+    all_f32 = all((vi.Y if vi.Y is not None else vi.model.Y).dtype == torch.float32 for vi in vis)
+    ydt = torch.float32 if all_f32 else f64
     for f, vi in enumerate(vis):
         if vi.r < 1 or vi.r > _lib.MAX_R:
             raise ValueError(f"latent_dim={vi.r} is outside the supported range 1..{_lib.MAX_R}")
@@ -566,7 +586,7 @@ def fit_batch(vis, max_iter: int = 100, tolerance: float = 1e-4, device=None, n_
             vi._engine.close()
             vi._engine = None
         cfg, kk = _fit_config(vi, dev.index)
-        Y = (vi.Y if vi.Y is not None else vi.model.Y).detach().to(dev, f64).contiguous()
+        Y = (vi.Y if vi.Y is not None else vi.model.Y).detach().to(dev, ydt).contiguous()
         src = vi._exact if (vi._exact is not None and vi._versions == (vi._host_mean._version, vi._host_cov._version)) else (vi._host_mean, vi._host_cov)
         Xm = src[0].detach().to(dev, f64).contiguous()
         Xc = src[1].detach().to(dev, f64).contiguous()
@@ -578,7 +598,8 @@ def fit_batch(vis, max_iter: int = 100, tolerance: float = 1e-4, device=None, n_
     ms = np.zeros((nf, max(max_iter, 1)))
     nd = (C.c_int32 * nf)()
     with torch.cuda.device(dev):
-        _lib.check(lib.tame_fit_batch(nf, cfgs, Yp, Mp, Cp, int(max_iter), float(tolerance), _lib.dptr(el), _lib.dptr(ms), nd, int(n_streams)))
+        batch = lib.tame_fit_batch_f32 if all_f32 else lib.tame_fit_batch
+        _lib.check(batch(nf, cfgs, Yp, Mp, Cp, int(max_iter), float(tolerance), _lib.dptr(el), _lib.dptr(ms), nd, int(n_streams)))
         torch.cuda.synchronize(dev)
     out = []
     for f, vi in enumerate(vis):

@@ -208,21 +208,26 @@ class TemporalAMEModel(StaticAMEModel):
         return X
 
     def generate_data_device(self, device="cuda", seed: int = 42, row_begin: int = 0, row_end: Optional[int] = None,
-                             keep_on_device: bool = True):
+                             keep_on_device: bool = True, dtype: torch.dtype = torch.float64):
         """Scalable generator: latents on the host (O(nTd)), observations written directly into HBM by the
         tame_generate_Y kernel (same distribution as temporal_ame.py:200-216, Philox keyed by (dyad, t)).
-        Returns rows [row_begin, row_end) of Y as a float64 CUDA tensor; `self.Y` is set to it (full rows only)."""
+        Returns rows [row_begin, row_end) of Y as a CUDA tensor of `dtype`; `self.Y` is set to it (full rows only).
+        dtype=torch.float32 computes in float64 and rounds once per value (tame_generate_Y_f32): half the HBM, and
+        the fits keep it as float32 on the device.  Other dtypes raise ValueError."""
         import ctypes as C
         from . import _lib
+        if dtype not in (torch.float64, torch.float32):
+            raise ValueError(f"generate_data_device: dtype must be torch.float64 or torch.float32, not {dtype}")
         lib = _lib.load()
+        gen = lib.tame_generate_Y_f32 if dtype == torch.float32 else lib.tame_generate_Y
         row_end = self.n if row_end is None else row_end
         dev = torch.device(device)
         self.X = self.generate_latents_fast(seed)
         Xd = self.X.to(dev)
-        Y = torch.empty(row_end - row_begin, self.n, self.T, 2, dtype=torch.float64, device=dev)
+        Y = torch.empty(row_end - row_begin, self.n, self.T, 2, dtype=dtype, device=dev)
         R = np.ascontiguousarray(self.R.double().numpy().reshape(4))
         with torch.cuda.device(dev):
-            _lib.check(lib.tame_generate_Y(self.n, self.T, self.r, _lib.dptr(R), Xd.data_ptr(), C.c_uint64(seed),
+            _lib.check(gen(self.n, self.T, self.r, _lib.dptr(R), Xd.data_ptr(), C.c_uint64(seed),
                                            row_begin, row_end, Y.data_ptr(),
                                            torch.cuda.current_stream(dev).cuda_stream))
             torch.cuda.synchronize(dev)
