@@ -106,6 +106,27 @@ class DeviceFit:
             self.h = C.c_void_p()
 
 
+class DeviceFit32(DeviceFit):
+    """DeviceFit with Y stored as float32 (a float32 CUDA tensor is used in place) and bound with tame_bind_Y_f32"""
+
+    def __init__(self, Y, Xm, Xc, c, lr, mode, device=0):
+        import torch
+        from tame_b200 import _lib
+        self._lib_mod = _lib
+        self.lib = _lib.load()
+        self.cfg, self._keep = make_config(c, lr, mode, device=device)
+        dev = torch.device("cuda", device)
+        self.Y = torch.as_tensor(np.ascontiguousarray(Y, dtype=np.float32)).to(dev) if not hasattr(Y, "data_ptr") else Y
+        self.Xm = torch.as_tensor(np.ascontiguousarray(Xm), dtype=torch.float64).to(dev) if not hasattr(Xm, "data_ptr") else Xm
+        self.Xc = torch.as_tensor(np.ascontiguousarray(Xc), dtype=torch.float64).to(dev) if not hasattr(Xc, "data_ptr") else Xc
+        torch.cuda.synchronize(dev)
+        self.h = C.c_void_p()
+        _lib.check(self.lib.tame_create(C.byref(self.cfg), C.byref(self.h)))
+        _lib.check(self.lib.tame_bind_Y_f32(self.h, self.Y.data_ptr()))
+        _lib.check(self.lib.tame_bind_state(self.h, self.Xm.data_ptr(), self.Xc.data_ptr()))
+        self.out = (C.c_double * 6)()
+
+
 def run_batch(fits, max_iter, tol, n_streams=0):
     """tame_fit_batch over `fits` = [(c, Y, Xm, Xc, lr, mode), ...] on fresh device copies of the state (Y may be a CUDA
     tensor already, shared by several fits).  Returns (traces, n_done, states, launches): traces[f] = (elbo, mse) cut at

@@ -13,7 +13,7 @@ import pytest
 import torch
 
 from conftest import GOLDEN_CASES, METHODS, golden_constants, load_golden
-from gpu_util import DeviceFit, fit_host, make_config, random_problem, run_batch
+from gpu_util import DeviceFit, DeviceFit32, fit_host, make_config, random_problem, run_batch
 from oracle import tame_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -35,26 +35,6 @@ def _lib():
 
 
 # ---- float32 counterparts of the gpu_util helpers (the float64 side uses gpu_util itself) -----------------------
-class DeviceFit32(DeviceFit):
-    """gpu_util.DeviceFit with Y stored as float32 and bound with tame_bind_Y_f32"""
-
-    def __init__(self, Y, Xm, Xc, c, lr, mode, device=0):
-        L = _lib()
-        self._lib_mod = L
-        self.lib = L.load()
-        self.cfg, self._keep = make_config(c, lr, mode, device=device)
-        dev = torch.device("cuda", device)
-        self.Y = torch.as_tensor(np.ascontiguousarray(Y, dtype=np.float32)).to(dev)
-        self.Xm = torch.as_tensor(np.ascontiguousarray(Xm), dtype=torch.float64).to(dev)
-        self.Xc = torch.as_tensor(np.ascontiguousarray(Xc), dtype=torch.float64).to(dev)
-        torch.cuda.synchronize(dev)
-        self.h = C.c_void_p()
-        L.check(self.lib.tame_create(C.byref(self.cfg), C.byref(self.h)))
-        L.check(self.lib.tame_bind_Y_f32(self.h, self.Y.data_ptr()))
-        L.check(self.lib.tame_bind_state(self.h, self.Xm.data_ptr(), self.Xc.data_ptr()))
-        self.out = (C.c_double * 6)()
-
-
 def fit_host32(Y, Xm, Xc, c, lr, mode, max_iter, tol=0.0):
     """gpu_util.fit_host through tame_fit_host_f32 (Y as float32 host memory)"""
     L = _lib()
